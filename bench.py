@@ -17,7 +17,8 @@ N > 1   : the factorisation does not shard (SURVEY.md 8e) -> "replicas only": ev
 reference arm: the UNMODIFIED reference (baseline/_ref, import shims only) through its own API on the host cores, timed
           at n in {1024, 2048, 4096, 8192}, fitted a n^3 + b n^2 and evaluated at n=32768 -- labelled extrapolated
           (a direct run is ~18 min and ~45 GB per evaluation, SURVEY 6); the oracle port if baseline/_ref is absent.
-One JSON line on stdout (rank 0).
+One JSON line on stdout (rank 0). --dump-outputs DIR: rank 0 also writes the NLL and gradient of its last timed step as
+          DIR/nll.npy and DIR/grad.npy (float64); the inputs are seeded, so runs with the same arguments compare directly.
 """
 import argparse
 import json
@@ -381,6 +382,8 @@ def run_ours(args):
                                    ctypes.byref(max_ms)), "profile read")
     nat.check(lib.gpk_profile(0), "profile off")
     clocks_rank = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"nll": np.array([last[0]], dtype=np.float64), "grad": last[1]})
     clocks_all = gather_obj(clocks_rank)
     clocks = clocks_all[0]
     t_dev = max_over_ranks(e0.elapsed_time(e1) * 1e-3)
@@ -724,6 +727,16 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(out_dir, arrays):
+    """What the timed path returned in its last step, one DIR/<name>.npy per array, so that two builds run with the
+    same arguments (hence the same seeded inputs) can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 _RESULT_FD = None
 
 
@@ -768,7 +781,13 @@ def main():
     ap.add_argument("--no-c2", action="store_true")
     ap.add_argument("--no-c5", action="store_true", help="skip the n=65536 d=32 leg (needs ~165 GB of HBM)")
     ap.add_argument("--no-dmma", action="store_true", help="skip the FP64-DMMA-only comparison leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's NLL and gradient as DIR/nll.npy, DIR/grad.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl ours)")
     _reserve_stdout()
     if args.impl == "reference":
         run_reference(args)

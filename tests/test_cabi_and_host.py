@@ -148,14 +148,14 @@ def test_crt_tables_are_current_and_self_consistent(tmp_path):
     import shutil
     hdr = os.path.join(PKG, "csrc", "oz_crt_tables.h")
     keep = tmp_path / "oz_crt_tables.h"
-    shutil.copy(hdr, keep)
+    shutil.copy2(hdr, keep)
     try:
         out = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "gen_crt_tables.py")], capture_output=True,
                              text=True)
         assert out.returncode == 0 and "CRT self-check ok" in out.stdout, out.stdout + out.stderr
         assert open(hdr).read() == open(keep).read(), "oz_crt_tables.h is stale: run tools/gen_crt_tables.py"
     finally:
-        shutil.copy(keep, hdr)
+        shutil.copy2(keep, hdr)    # with its mtime, or build_native would take libgpk.so for stale and rebuild it
     # moduli: pairwise coprime, <= 256, and 17 of them carry 58-bit operands at K = 32768
     from math import gcd, log2
     mods = [256, 255, 253, 251, 247, 241, 239, 233, 229, 227, 223, 217, 211, 199, 197, 193, 191, 181]
@@ -200,22 +200,31 @@ def test_bench_reference_arm_prints_one_json_line():
     assert res.returncode == 0 and res.stdout.strip() == ""
 
 
-def test_reference_arm_port_and_install_agree(tmp_path):
-    """The oracle port (used when baseline/_ref is absent) and the installed reference give the same NLL / gradient on
-    the bench workload: the two `kind`s of the reference arm time the same computation."""
-    if not os.path.isdir(os.path.join(ROOT, "baseline", "_ref", "skgpuppy")):
-        pytest.skip("reference not installed in baseline/_ref")
-    code = ("import sys, json; sys.path.insert(0, %r); import bench; import numpy as np\n"
-            "f, g, kind = bench._reference_callables()\n"
-            "x, t, th = bench.synthetic(300, 5, 7)\n"
-            "print(json.dumps([kind, float(f(x, t, th)), [float(v) for v in g(x, t, th)]]))" % ROOT)
-    res = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
-    assert res.returncode == 0, res.stderr[-2000:]
+def test_reference_arm_port_and_install_agree(golden):
+    """Whichever `kind` the reference arm uses (the oracle port, or the installed reference in baseline/_ref), it gives
+    the unmodified reference's NLL / gradient on the bench workload: tests/golden/syn_*.npz hold the reference's own
+    values on the inputs bench.synthetic draws for these seeds (oracle/make_golden.py)."""
     import json
-    kind, nll, grad = json.loads(res.stdout.strip().splitlines()[-1])
-    assert kind == "reference"
     sys.path.insert(0, ROOT)
     import bench
-    x, t, th = bench.synthetic(300, 5, 7)
-    assert nll == pytest.approx(O.negativeloglikelihood(x, t, th), rel=1e-12)
-    np.testing.assert_allclose(grad, O.d_nll_d_theta(x, t, th), rtol=1e-10)
+    cases = [("syn_n512_d8", 512, 8, 2003), ("syn_n384_d16", 384, 16, 2004)]
+    for name, n, d, seed in cases:
+        g = golden(name)
+        x, t, th = bench.synthetic(n, d, seed)
+        assert np.array_equal(x, g["x"]) and np.array_equal(t, g["t"] - g["t"].mean()) and np.array_equal(th, g["theta"])
+    code = ("import sys, json; sys.path.insert(0, %r); import bench; import numpy as np\n"
+            "f, g, kind = bench._reference_callables()\n"
+            "out = [kind]\n"
+            "for n, d, seed in %r:\n"
+            "    x, t, th = bench.synthetic(n, d, seed)\n"
+            "    out.append([float(f(x, t, th)), [float(v) for v in g(x, t, th)]])\n"
+            "print(json.dumps(out))" % (ROOT, [c[1:] for c in cases]))
+    res = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
+    assert res.returncode == 0, res.stderr[-2000:]
+    out = json.loads(res.stdout.strip().splitlines()[-1])
+    installed = os.path.isdir(os.path.join(ROOT, "baseline", "_ref", "skgpuppy"))
+    assert out[0] == ("reference" if installed else "port")
+    for (name, _, _, _), (nll, grad) in zip(cases, out[1:]):
+        g = golden(name)
+        assert nll == pytest.approx(float(g["nll"]), rel=1e-12), name
+        np.testing.assert_allclose(grad, g["grad"], rtol=1e-10, err_msg=name)
