@@ -12,18 +12,9 @@
 extern "C" {
 #endif
 
-/* FP64 DMMA GEMM: C = beta*C + alpha * A(m,k) B(n,k) over the per-tile k range; layouts 0 = k contiguous, 1 = m/n
- * contiguous; epi 0 = store (128x128 tile), 1 = column squares, 2 / 4 / 5 = store with 64x64 / 64x32 / 64x128 tiles. */
-int gpk_test_gemm(int alay, int blay, int epi, const double* A_dev, int64_t lda, const double* B_dev, int64_t ldb,
-                  double* C_dev, int64_t ldc, int64_t M, int64_t N, int64_t K, double alpha, double beta, int krange,
-                  int lower_only, double* colsq_dev, double* pairdot_dev, int64_t ldo, void* cuda_stream);
-
 /* In: A (lower tiles of an SPD matrix, order npad, ld). Out: X = L^-1, dL = diag(L), *info_host (0 = ok). FP64 DMMA. */
 int gpk_test_potrf_inv(double* A_dev, double* X_dev, int64_t ld, int64_t npad, double* dL_dev, int* info_host,
                        void* cuda_stream);
-
-/* out = X^T X (lower tiles). FP64 DMMA. */
-int gpk_test_lauum(const double* X_dev, double* out_dev, int64_t ld, int64_t npad, void* cuda_stream);
 
 /*
  * FP64 GEMM through the INT8 tcgen05 tensor cores (csrc/oz_gemm.cuh).
@@ -40,10 +31,6 @@ int gpk_test_oz_gemm(const double* A_dev, int64_t lda, int transA, int lowerA, c
                      int transB, int lowerB, double* C_dev, int64_t ldc, int64_t M, int64_t N, int64_t K, double alpha,
                      double beta, int krange, int lower_only, int moduli, int64_t panel_rows, int reps,
                      float* ms_out_host, void* cuda_stream);
-
-/* Tuning experiments (calling thread only): CTA raster band height of the planes kernel (pair rows, > 0) and warps per
- * row of the reconstruction kernel (1, 2, 4). 0 / other values leave a setting unchanged. */
-int gpk_test_tune(int group_m, int recon_cw);
 
 /* Planes kernel (calling thread only): 0 = a CTA pair that starts a tile adopts the modulus of the most advanced pair and
  * starts at its first k-block; 1 = it adopts the (modulus, k-block) position, splitting its first modulus; 2 = in
@@ -65,9 +52,6 @@ int gpk_test_overlap(int on);
 int gpk_profile(int on);
 int gpk_profile_read(double* gemm_ms_host, int64_t* gemm_launches_host, int64_t* all_launches_host,
                      double* max_gemm_ms_host);
-
-/* Register-resident FP64 throughput probes: kind 0 = DMMA.8x8x4, 1 = DFMA. Returns TFLOP/s in *out_host. */
-int gpk_microbench(int kind, int64_t iters, double* out_host);
 
 /*
  * INT8 tensor-pipe peak of this GPU: every SM pair issues tcgen05.mma.cta_group::2.kind::i8 (M = 256, N = 256, K = 32)

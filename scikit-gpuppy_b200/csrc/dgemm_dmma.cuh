@@ -68,9 +68,7 @@ struct GemmArgs {
   int krange;
   int lower_only;   // skip tiles entirely above the diagonal
   int reverse_bi;   // schedule large bi first (heavy-first for K_UPTO_BI)
-  int group_m;      // > 0: CTA raster swizzle, consecutive CTAs sweep column-major through bands of group_m tile rows
   double* colsq; double* pairdot; long ldo;  // EPI_COLSQ outputs: colsq[bi*ldo + n], pairdot[bi*(ldo/2) + n/2]
-  long strideA, strideB, strideC;            // blockIdx.z batching
 };
 
 __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src) {
@@ -113,20 +111,17 @@ __global__ void __launch_bounds__(T::THREADS, T::MINCTAS) dgemm_dmma_kernel(Gemm
   pdl_wait();
   const int tid = threadIdx.x;
   // Raster: the CTAs resident at one time (148 x MINCTAS) should share as few A/B panels as possible, so the
-  // linear CTA id walks column-major through bands of group_m tile rows (a near-square working set) instead of
+  // linear CTA id walks column-major through bands of GROUP_M tile rows (a near-square working set) instead of
   // along whole tile rows. ncu on 8192^3: DRAM reads 64 GB row-major vs the 1.6 GB the operands occupy.
-  int bx = blockIdx.x, by = blockIdx.y;
-  if (p.group_m > 0) {
-    const int pid = by * gridDim.x + bx;
-    const int per_band = p.group_m * gridDim.x;
-    const int band = pid / per_band;
-    const int first = band * p.group_m;
-    const int rows = min((int)gridDim.y - first, p.group_m);
-    const int rem = pid - band * per_band;
-    by = first + rem % rows;
-    bx = rem / rows;
-  }
-  const int bj = bx;
+  constexpr int GROUP_M = (TM >= 128) ? 8 : 16;   // band height in tile rows
+  const int pid = blockIdx.y * gridDim.x + blockIdx.x;
+  const int per_band = GROUP_M * gridDim.x;
+  const int band = pid / per_band;
+  const int first = band * GROUP_M;
+  const int rows = min((int)gridDim.y - first, GROUP_M);
+  const int rem = pid - band * per_band;
+  const int by = first + rem % rows;
+  const int bj = rem / rows;
   const int bi = p.reverse_bi ? (gridDim.y - 1 - by) : by;
   if (p.lower_only && bj * TN > bi * TM + (TM - 1)) return;
 
@@ -141,9 +136,6 @@ __global__ void __launch_bounds__(T::THREADS, T::MINCTAS) dgemm_dmma_kernel(Gemm
     default: break;
   }
   const int nk = (ke - kb) / GEMM_BK;
-
-  const double* A = p.A + blockIdx.z * p.strideA;
-  const double* B = p.B + blockIdx.z * p.strideB;
 
   double* As = smem;
   double* Bs = smem + STAGES * T::A_ELEMS;
@@ -170,10 +162,10 @@ __global__ void __launch_bounds__(T::THREADS, T::MINCTAS) dgemm_dmma_kernel(Gemm
     if (s < nk) {
 #pragma unroll
       for (int r = 0; r < T::PA; ++r)
-        load_chunk_part<ALAY, TM, T::THREADS>(As + s * T::A_ELEMS, A, p.lda, bi * TM, kb + s * GEMM_BK, tid, r);
+        load_chunk_part<ALAY, TM, T::THREADS>(As + s * T::A_ELEMS, p.A, p.lda, bi * TM, kb + s * GEMM_BK, tid, r);
 #pragma unroll
       for (int r = 0; r < T::PB; ++r)
-        load_chunk_part<BLAY, TN, T::THREADS>(Bs + s * T::B_ELEMS, B, p.ldb, bj * TN, kb + s * GEMM_BK, tid, r);
+        load_chunk_part<BLAY, TN, T::THREADS>(Bs + s * T::B_ELEMS, p.B, p.ldb, bj * TN, kb + s * GEMM_BK, tid, r);
     }
     cp_async_commit();
   }
@@ -220,10 +212,10 @@ __global__ void __launch_bounds__(T::THREADS, T::MINCTAS) dgemm_dmma_kernel(Gemm
       if (do_load) {
 #pragma unroll
         for (int r = (ks * T::PA) / 4; r < ((ks + 1) * T::PA) / 4; ++r)
-          load_chunk_part<ALAY, TM, T::THREADS>(as_n, A, p.lda, bi * TM, k_n, tid, r);
+          load_chunk_part<ALAY, TM, T::THREADS>(as_n, p.A, p.lda, bi * TM, k_n, tid, r);
 #pragma unroll
         for (int r = (ks * T::PB) / 4; r < ((ks + 1) * T::PB) / 4; ++r)
-          load_chunk_part<BLAY, TN, T::THREADS>(bs_n, B, p.ldb, bj * TN, k_n, tid, r);
+          load_chunk_part<BLAY, TN, T::THREADS>(bs_n, p.B, p.ldb, bj * TN, k_n, tid, r);
       }
 #pragma unroll
       for (int i = 0; i < 4; ++i)
@@ -235,7 +227,6 @@ __global__ void __launch_bounds__(T::THREADS, T::MINCTAS) dgemm_dmma_kernel(Gemm
   cp_async_wait<0>();
 
   if (EPI == EPI_STORE) {
-    double* C = p.C + blockIdx.z * p.strideC;
     const double alpha = p.alpha, beta = p.beta;
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
@@ -243,7 +234,7 @@ __global__ void __launch_bounds__(T::THREADS, T::MINCTAS) dgemm_dmma_kernel(Gemm
 #pragma unroll
       for (int j = 0; j < NJ; ++j) {
         const long col = (long)bj * TN + wn * (TN / 2) + j * 8 + 2 * tg;
-        double2* ptr = reinterpret_cast<double2*>(C + row * p.ldc + col);
+        double2* ptr = reinterpret_cast<double2*>(p.C + row * p.ldc + col);
         double2 v;
         v.x = alpha * acc[i][j][0];
         v.y = alpha * acc[i][j][1];
@@ -302,7 +293,7 @@ __global__ void __launch_bounds__(T::THREADS, T::MINCTAS) dgemm_dmma_kernel(Gemm
 }
 
 template <int ALAY, int BLAY, int EPI, class T = Tile128>
-inline int gemm_launch(const GemmArgs& a, int batch, cudaStream_t st) {
+inline int gemm_launch(const GemmArgs& a, cudaStream_t st) {
   static bool configured_on[GPK_MAX_DEVICES] = {};
   bool& configured = configured_on[current_device_slot()];
   if (!configured) {
@@ -315,17 +306,14 @@ inline int gemm_launch(const GemmArgs& a, int batch, cudaStream_t st) {
     snprintf(g_err, sizeof(g_err), "gemm_launch: extents %d,%d,%d not tile multiples", a.M, a.N, a.K);
     return -2;
   }
-  dim3 grid(a.N / T::TN, a.M / T::TM, batch);
-  GemmArgs aa = a;
-  if (aa.group_m < 0) aa.group_m = 0;
-  else if (aa.group_m == 0) aa.group_m = (T::TM >= 128) ? 8 : 16;   // default band height in tile rows
+  dim3 grid(a.N / T::TN, a.M / T::TM);
   cudaEvent_t e0 = nullptr, e1 = nullptr;
   if (g_prof_on) {
     GPK_CUDA_OK(cudaEventCreate(&e0));
     GPK_CUDA_OK(cudaEventCreate(&e1));
     GPK_CUDA_OK(cudaEventRecord(e0, st));
   }
-  GPK_CUDA_OK(launch_pdl(dgemm_dmma_kernel<ALAY, BLAY, EPI, T>, grid, dim3(T::THREADS), (size_t)T::SMEM_BYTES, st, aa));
+  GPK_CUDA_OK(launch_pdl(dgemm_dmma_kernel<ALAY, BLAY, EPI, T>, grid, dim3(T::THREADS), (size_t)T::SMEM_BYTES, st, a));
   GPK_LAUNCH_OK();
   if (g_prof_on) {
     GPK_CUDA_OK(cudaEventRecord(e1, st));
@@ -340,13 +328,13 @@ template <int ALAY, int BLAY>
 inline int gemm_store_auto(const GemmArgs& a, cudaStream_t st) {
   long tiles = (long)(a.M / 64) * (a.N / 128);
   if (a.lower_only) tiles /= 2;
-  if (tiles >= 2 * 2 * 148) return gemm_launch<ALAY, BLAY, EPI_STORE, Tile64x128>(a, 1, st);
+  if (tiles >= 2 * 2 * 148) return gemm_launch<ALAY, BLAY, EPI_STORE, Tile64x128>(a, st);
   // sub-2048 nodes of the recursion: 64x64 tiles leave 1.7 CTAs per SM at order 1024 and 4-64 CTAs in all below;
   // 64x32 tiles (4 CTAs/SM) double the CTA count for the same work: 16.9 -> 12.2 ms of small GEMMs per fit iteration at
   // n = 32768, 2.0 -> 1.45 ms at n = 4096 (32x32 tiles measured the same as 64x32)
   const long t64 = (long)(a.M / 64) * (a.N / 64);
-  if (t64 <= 512) return gemm_launch<ALAY, BLAY, EPI_STORE, GemmTile<64, 32, 4, 4>>(a, 1, st);
-  return gemm_launch<ALAY, BLAY, EPI_STORE, Tile64>(a, 1, st);
+  if (t64 <= 512) return gemm_launch<ALAY, BLAY, EPI_STORE, GemmTile<64, 32, 4, 4>>(a, st);
+  return gemm_launch<ALAY, BLAY, EPI_STORE, Tile64>(a, st);
 }
 
 inline GemmArgs gemm_args(const double* A, long lda, const double* B, long ldb, double* C, long ldc,

@@ -407,39 +407,10 @@ static int quad_forms(Handle* h, long rows) {
   a.colsq = h->colsq;
   a.pairdot = h->pairdot;
   a.ldo = rows;
-  return gemm_launch<LAY_KC, LAY_KC, EPI_COLSQ>(a, 1, h->st);
+  return gemm_launch<LAY_KC, LAY_KC, EPI_COLSQ>(a, h->st);
 }
 
 // ---- microbenchmarks -----------------------------------------------------------------------
-__global__ void __launch_bounds__(256) mb_dmma_kernel(long iters, double* out) {
-  double c[16][2];
-#pragma unroll
-  for (int i = 0; i < 16; ++i) c[i][0] = c[i][1] = 0.0;
-  double a = 1.0 + threadIdx.x * 1e-9, b = 1.0 - threadIdx.x * 1e-9;
-  for (long it = 0; it < iters; ++it) {
-#pragma unroll
-    for (int i = 0; i < 16; ++i) dmma884(c[i][0], c[i][1], a, b);
-  }
-  double s = 0.0;
-#pragma unroll
-  for (int i = 0; i < 16; ++i) s += c[i][0] + c[i][1];
-  if (s == 123.456) out[0] = s;
-}
-__global__ void __launch_bounds__(256) mb_dfma_kernel(long iters, double* out) {
-  double c[16];
-#pragma unroll
-  for (int i = 0; i < 16; ++i) c[i] = i;
-  double a = 1.0 + threadIdx.x * 1e-9, b = 1e-9;
-  for (long it = 0; it < iters; ++it) {
-#pragma unroll
-    for (int i = 0; i < 16; ++i) c[i] = fma(c[i], a, b);
-  }
-  double s = 0.0;
-#pragma unroll
-  for (int i = 0; i < 16; ++i) s += c[i];
-  if (s == 123.456) out[0] = s;
-}
-
 // INT8 tensor-pipe probe: one CTA pair per two SMs, tcgen05.mma.cta_group::2.kind::i8 M=256 N=256 K=32 issued back to
 // back from shared-memory tiles filled with pseudo-random bytes (so the datapath toggles like real operands), two
 // 256-column TMEM accumulators alternating. No TMA, no epilogue: the ceiling of oz_crt_planes_kernel's MMA stream.
@@ -1117,33 +1088,6 @@ int gpk_propagate_ga_parts(gpk_handle h, const double* U, const double* S, int64
 }
 
 // ---- test / measurement hooks --------------------------------------------------------------
-int gpk_test_gemm(int alay, int blay, int epi, const double* A, int64_t lda, const double* B, int64_t ldb, double* C,
-                  int64_t ldc, int64_t M, int64_t N, int64_t K, double alpha, double beta, int krange, int lower_only,
-                  double* colsq, double* pairdot, int64_t ldo, void* stream) {
-  GemmArgs a = gemm_args(A, lda, B, ldb, C, ldc, (int)M, (int)N, (int)K, alpha, beta, krange, lower_only);
-  a.colsq = colsq; a.pairdot = pairdot; a.ldo = ldo;
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const int key = alay * 100 + blay * 10 + epi;
-  switch (key) {
-    // epi 0 / 1: the production store / column-square epilogues (128x128 tile); 2, 4, 5: the store epilogue with the
-    // other CTA tiles the factorisation picks (64x64, 64x32, 64x128)
-    case 0: return gemm_launch<LAY_KC, LAY_KC, EPI_STORE>(a, 1, st);
-    case 1: return gemm_launch<LAY_KC, LAY_KC, EPI_COLSQ>(a, 1, st);
-    case 10: return gemm_launch<LAY_KC, LAY_MC, EPI_STORE>(a, 1, st);
-    case 110: return gemm_launch<LAY_MC, LAY_MC, EPI_STORE>(a, 1, st);
-    case 2: return gemm_launch<LAY_KC, LAY_KC, EPI_STORE, Tile64>(a, 1, st);
-    case 12: return gemm_launch<LAY_KC, LAY_MC, EPI_STORE, Tile64>(a, 1, st);
-    case 112: return gemm_launch<LAY_MC, LAY_MC, EPI_STORE, Tile64>(a, 1, st);
-    case 4: return gemm_launch<LAY_KC, LAY_KC, EPI_STORE, GemmTile<64, 32, 4, 4>>(a, 1, st);
-    case 5: return gemm_launch<LAY_KC, LAY_KC, EPI_STORE, Tile64x128>(a, 1, st);
-    case 15: return gemm_launch<LAY_KC, LAY_MC, EPI_STORE, Tile64x128>(a, 1, st);
-    case 115: return gemm_launch<LAY_MC, LAY_MC, EPI_STORE, Tile64x128>(a, 1, st);
-    default:
-      snprintf(g_err, sizeof(g_err), "gpk_test_gemm: variant %d not instantiated", key);
-      return -2;
-  }
-}
-
 int gpk_test_potrf_inv(double* A, double* X, int64_t ld, int64_t npad, double* dL, int* info_host, void* stream) {
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   if (npad % TILE) { snprintf(g_err, sizeof(g_err), "npad must be a multiple of 128"); return -2; }
@@ -1160,10 +1104,6 @@ int gpk_test_potrf_inv(double* A, double* X, int64_t ld, int64_t npad, double* d
   if (e != cudaSuccess) { snprintf(g_err, sizeof(g_err), "potrf_inv: %s", cudaGetErrorString(e)); return -1; }
   *info_host = (info == INT_MAX) ? 0 : info;
   return 0;
-}
-
-int gpk_test_lauum(const double* X, double* out, int64_t ld, int64_t npad, void* stream) {
-  return lauum_launch(X, out, ld, (int)npad, reinterpret_cast<cudaStream_t>(stream), nullptr);
 }
 
 int gpk_test_oz_residues(const double* src, int64_t ld, int64_t rows, int64_t K, int trans, int lower, int moduli,
@@ -1240,12 +1180,6 @@ int gpk_test_oz_gemm(const double* A, int64_t lda, int transA, int lowerA, const
   }
 #undef OZ_OK
   cleanup();
-  return 0;
-}
-
-int gpk_test_tune(int group_m, int recon_cw) {
-  if (group_m > 0) oz::g_group_m = group_m;
-  if (recon_cw == 1 || recon_cw == 2 || recon_cw == 4) oz::g_recon_cw = recon_cw;
   return 0;
 }
 
@@ -1343,31 +1277,6 @@ int gpk_microbench_i8(int64_t iters, double seconds, double* out_host) {
     out_host[1] = ops_per_launch * launches / (ms * 1e-3) / 1e12;
   }
   cudaEventDestroy(e0); cudaEventDestroy(e1);
-  return 0;
-}
-
-int gpk_microbench(int kind, int64_t iters, double* out_host) {
-  double* dev = nullptr;
-  GPK_CUDA_OK(cudaMalloc((void**)&dev, sizeof(double)));
-  int nsm = 0;
-  GPK_CUDA_OK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, 0));
-  cudaEvent_t e0, e1;
-  GPK_CUDA_OK(cudaEventCreate(&e0));
-  GPK_CUDA_OK(cudaEventCreate(&e1));
-  const int blocks = nsm * 4;
-  for (int rep = 0; rep < 2; ++rep) {
-    GPK_CUDA_OK(cudaEventRecord(e0));
-    if (kind == 0) mb_dmma_kernel<<<blocks, 256>>>(iters, dev);
-    else mb_dfma_kernel<<<blocks, 256>>>(iters, dev);
-    GPK_CUDA_OK(cudaEventRecord(e1));
-    GPK_CUDA_OK(cudaEventSynchronize(e1));
-  }
-  float ms = 0.f;
-  GPK_CUDA_OK(cudaEventElapsedTime(&ms, e0, e1));
-  const double warps = (double)blocks * 8.0;
-  const double flops = (kind == 0) ? warps * iters * 16.0 * 512.0 : warps * 32.0 * iters * 16.0 * 2.0;
-  *out_host = flops / (ms * 1e-3) / 1e12;
-  cudaEventDestroy(e0); cudaEventDestroy(e1); cudaFree(dev);
   return 0;
 }
 

@@ -16,7 +16,7 @@ struct PlaneArgs {
   uint8_t* res; long res_ld; long res_plane;   // residue planes [nmod][panel rows][res_ld] (one byte per element)
   int M, N, K;
   int row_tile0;                               // first 256-row tile of this row panel
-  int krange, lower_only, group_m;
+  int krange, lower_only;
   int widen, band_cols;                        // band-uniform k ranges; raster bands over columns instead of rows
   int nmod;
   unsigned int* phase;                         // position (modulus step, k-block) of the most advanced CTA pair of the launch
@@ -33,7 +33,6 @@ struct ReconArgs {
   double alpha, beta;
   int M, N, K;
   int row0;                                    // first row of this panel (multiple of 256)
-  long ncols_pad;                              // 128-column blocks this launch covers, in columns
   int krange, lower_only;
   int nmod;
   double p_scaled;                             // P * 2^-96
@@ -69,32 +68,30 @@ oz_crt_planes_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
   const uint32_t rank = cluster_ctarank();
   const int pp = (int)(rank & 1u);            // CTA within its pair: M half of the tile and N half of the B rows it loads
 
-  int bx = blockIdx.x >> 1, by = blockIdx.y;
   const int nx = gridDim.x >> 1, ny = (int)gridDim.y;
-  int band_lo = 0, band_hi = 0;               // first / last pair row (or column) of this tile's raster band
-  if (p.group_m > 0) {
-    const int pid = by * nx + bx;
-    if (!p.band_cols) {                       // bands of group_m pair rows, column-major inside a band
-      const int per_band = p.group_m * nx;
-      const int band = pid / per_band;
-      const int first = band * p.group_m;
-      const int rows = min(ny - first, p.group_m);
-      const int rem = pid - band * per_band;
-      by = first + rem % rows;
-      bx = rem / rows;
-      band_lo = first + p.row_tile0;
-      band_hi = first + rows - 1 + p.row_tile0;
-    } else {                                  // bands of group_m pair columns, row-major inside a band
-      const int per_band = p.group_m * ny;
-      const int band = pid / per_band;
-      const int first = band * p.group_m;
-      const int cols = min(nx - first, p.group_m);
-      const int rem = pid - band * per_band;
-      bx = first + rem % cols;
-      by = rem / cols;
-      band_lo = first;
-      band_hi = first + cols - 1;
-    }
+  const int pid = (int)blockIdx.y * nx + (int)(blockIdx.x >> 1);
+  int bx, by;
+  int band_lo, band_hi;                       // first / last pair row (or column) of this tile's raster band
+  if (!p.band_cols) {                         // bands of PLANES_BAND pair rows, column-major inside a band
+    const int per_band = PLANES_BAND * nx;
+    const int band = pid / per_band;
+    const int first = band * PLANES_BAND;
+    const int rows = min(ny - first, PLANES_BAND);
+    const int rem = pid - band * per_band;
+    by = first + rem % rows;
+    bx = rem / rows;
+    band_lo = first + p.row_tile0;
+    band_hi = first + rows - 1 + p.row_tile0;
+  } else {                                    // bands of PLANES_BAND pair columns, row-major inside a band
+    const int per_band = PLANES_BAND * ny;
+    const int band = pid / per_band;
+    const int first = band * PLANES_BAND;
+    const int cols = min(nx - first, PLANES_BAND);
+    const int rem = pid - band * per_band;
+    bx = first + rem % cols;
+    by = rem / cols;
+    band_lo = first;
+    band_hi = first + cols - 1;
   }
   const int bi2 = by + p.row_tile0;           // global pair-row tile
   const int bi = 2 * bi2 + pp;                // 128-row tile of A this CTA loads
@@ -325,17 +322,13 @@ __device__ __forceinline__ uint32_t dp2a_hi(uint32_t a, uint32_t b, uint32_t c) 
 }
 
 // NG = groups of 4 moduli (compile time: no per-plane predicates or index multiplies for the groups that are full).
-// CW = warps side by side in a row: a block covers (8 / CW) rows x (128 CW) columns, so that each (plane, row) read is
-// 128 CW contiguous bytes and each FP64 row write 1 KB x CW (DRAM page locality of 16 planes x rows far apart).
-template <int EPI, int NG, int CW>
+// Blocks of 2 or 4 warps side by side in a row (longer contiguous reads and writes per row) made no measurable
+// difference (profiles/r2_tune_planes.txt).
+template <int EPI, int NG>
 __global__ void __launch_bounds__(256, 4) oz_crt_reconstruct_kernel(const __grid_constant__ ReconArgs p) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int bjc = blockIdx.x * CW + (warp % CW);                // 128-column block
-  const long lrow = (long)blockIdx.y * (8 / CW) + warp / CW;
-  if ((long)bjc * 128 >= p.ncols_pad) {                         // odd number of 128-column blocks: idle warp
-    if (EPI != OZ_EPI_STORE) __syncthreads();
-    return;
-  }
+  const int bjc = blockIdx.x;                                   // 128-column block
+  const long lrow = (long)blockIdx.y * 8 + warp;
   const long grow = (long)p.row0 + lrow;
   const long gcol = (long)bjc * 128 + lane * 4;
   const int bi = (int)(grow >> 7), bi2 = (int)(grow >> 8), bx2 = bjc >> 1;
@@ -417,7 +410,7 @@ __global__ void __launch_bounds__(256, 4) oz_crt_reconstruct_kernel(const __grid
 #pragma unroll
     for (int x = 0; x < 4; ++x) {
       sq = fma(v[x], v[x], sq);
-      pd = fma(v[x], vrow[warp ^ CW][lane * 4 + x], pd);
+      pd = fma(v[x], vrow[warp ^ 1][lane * 4 + x], pd);
     }
 #pragma unroll
     for (int off = 1; off < 32; off <<= 1) {

@@ -184,7 +184,10 @@ __device__ __forceinline__ bool oz_valid(int r, int k, int lower) {
 // ranges, 1 + WIDEN_TILES when the product is long enough (K >= WIDEN_MIN_K) for the planes kernel to give every tile
 // of a raster band the same k range (see oz_crt_planes_kernel: tiles in step share their operand panels in L2).
 constexpr int WIDEN_MIN_K = 16384;   // at K = 8192 the added k-blocks and zero tiles cost more than the sharing saves (propagate_GA -3 %)
-constexpr int WIDEN_TILES = 6;     // (band height 4 - 1) pair rows = 6 k-blocks
+// CTA raster of the planes kernel: consecutive CTA pairs sweep bands of PLANES_BAND pair rows (or pair columns). Bands
+// of 2 / 6 / 8 / 16 ran 6-22 % slower on the K^-1 launch at n = 32768 (profiles/r2_tune_planes.txt).
+constexpr int PLANES_BAND = 4;
+constexpr int WIDEN_TILES = 2 * (PLANES_BAND - 1);   // k-blocks between the first and the last pair row of a band
 inline int zero_fill_extra(int K) { return K >= WIDEN_MIN_K ? 1 + WIDEN_TILES : 1; }
 template <int TRANS>
 __device__ __forceinline__ bool oz_needed(int r, int k, int lower, int extra) {
@@ -444,11 +447,7 @@ inline int slice_operand(const double* src, long ld, int trans, int lower, Opera
   return 0;
 }
 
-// CTA raster of the planes kernel: column-major through bands of g_group_m pair rows; block shape of the reconstruction
-// kernel. Compile-time defaults; gpk_test_tune (include/gpk_test.h) changes them for the calling thread in experiments.
 thread_local int g_position_lock = 2;   // gpk_test_position_lock: 0 = lock on the modulus only, 1 = + split first modulus, 2 = + band-uniform k ranges
-thread_local int g_group_m = 4;
-thread_local int g_recon_cw = 1;
 
 // C = beta*C + alpha * A * B^T over the per-tile k range, from operands in residue form (A.K == B.K, A.S == B.S):
 // per row panel that fits A.out, one GEMM launch (all moduli) and one reconstruction launch.
@@ -485,9 +484,8 @@ inline int gemm_sliced(const Operand& A, const Operand& B, double* C, long ldc, 
   memset(&g, 0, sizeof(g));
   g.res = A.out; g.res_ld = Nc;
   g.M = A.rows; g.N = B.rows; g.K = A.K; g.krange = krange; g.lower_only = lower_only; g.nmod = A.S;
-  g.group_m = g_group_m;
   // band-uniform k ranges (and column bands for the column-dependent ranges) when the operands are far larger than L2
-  g.widen = (g_position_lock >= 2 && g.group_m > 0 && g.group_m <= 4 && A.K >= WIDEN_MIN_K &&
+  g.widen = (g_position_lock >= 2 && A.K >= WIDEN_MIN_K &&
              (krange == K_FROM_BI || krange == K_UPTO_BI || krange == K_FROM_BJ || krange == K_UPTO_BJ)) ? 1 : 0;
   g.band_cols = (g.widen && (krange == K_FROM_BJ || krange == K_UPTO_BJ)) ? 1 : 0;
   ReconArgs r;
@@ -551,27 +549,14 @@ inline int gemm_sliced(const Operand& A, const Operand& B, double* C, long ldc, 
     GPK_LAUNCH_OK();
     long ncol_blocks = B.rows / 128;
     if (lower_only && (row0 + rows) / 128 < ncol_blocks) ncol_blocks = (row0 + rows) / 128;
-    r.ncols_pad = ncol_blocks * 128;
-    const int cw = g_recon_cw;             // warps side by side per row (1, 2 or 4); rows are multiples of 8
-    dim3 rg((unsigned)((ncol_blocks + cw - 1) / cw), (unsigned)(rows / (8 / cw)));
+    dim3 rg((unsigned)ncol_blocks, (unsigned)(rows / 8));   // rows are multiples of 8
     const int ng = (A.S + 3) / 4;      // 2..RECON_GROUPS
-#define GPK_RECON2(NG, CW)                                                                           \
-  do {                                                                                               \
-    if (epi == OZ_EPI_STORE) oz_crt_reconstruct_kernel<OZ_EPI_STORE, NG, CW><<<rg, 256, 0, st>>>(r); \
-    else oz_crt_reconstruct_kernel<OZ_EPI_ROWSQ, NG, CW><<<rg, 256, 0, st>>>(r);                     \
-  } while (0)
-#define GPK_RECON(NG)                       \
-  do {                                      \
-    if (cw == 1) GPK_RECON2(NG, 1);         \
-    else if (cw == 2) GPK_RECON2(NG, 2);    \
-    else GPK_RECON2(NG, 4);                 \
-  } while (0)
-    if (ng <= 2) GPK_RECON(2);
-    else if (ng == 3) GPK_RECON(3);
-    else if (ng == 4) GPK_RECON(4);
-    else GPK_RECON(5);
-#undef GPK_RECON
-#undef GPK_RECON2
+    const bool store = epi == OZ_EPI_STORE;
+    auto kernel = (ng <= 2) ? (store ? oz_crt_reconstruct_kernel<OZ_EPI_STORE, 2> : oz_crt_reconstruct_kernel<OZ_EPI_ROWSQ, 2>)
+                : (ng == 3) ? (store ? oz_crt_reconstruct_kernel<OZ_EPI_STORE, 3> : oz_crt_reconstruct_kernel<OZ_EPI_ROWSQ, 3>)
+                : (ng == 4) ? (store ? oz_crt_reconstruct_kernel<OZ_EPI_STORE, 4> : oz_crt_reconstruct_kernel<OZ_EPI_ROWSQ, 4>)
+                            : (store ? oz_crt_reconstruct_kernel<OZ_EPI_STORE, 5> : oz_crt_reconstruct_kernel<OZ_EPI_ROWSQ, 5>);
+    kernel<<<rg, 256, 0, st>>>(r);
     GPK_LAUNCH_OK();
   }
   if (g_prof_on) {

@@ -52,21 +52,15 @@ SIGNATURES = {
 
 # measurement / test hooks (include/gpk_test.h): bound for tests/ and bench.py, never called by the product layer
 TEST_SIGNATURES = {
-    "gpk_test_gemm": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.c_int, vp, i64, vp, i64, vp, i64, i64, i64,
-                                     i64, ctypes.c_double, ctypes.c_double, ctypes.c_int, ctypes.c_int, vp, vp, i64,
-                                     vp]),
     "gpk_test_potrf_inv": (ctypes.c_int, [vp, vp, i64, i64, vp, c_int_p, vp]),
-    "gpk_test_lauum": (ctypes.c_int, [vp, vp, i64, i64, vp]),
     "gpk_test_oz_residues": (ctypes.c_int, [vp, i64, i64, i64, ctypes.c_int, ctypes.c_int, ctypes.c_int, vp, vp, vp]),
     "gpk_test_oz_gemm": (ctypes.c_int, [vp, i64, ctypes.c_int, ctypes.c_int, vp, i64, ctypes.c_int, ctypes.c_int, vp, i64,
                                         i64, i64, i64, ctypes.c_double, ctypes.c_double, ctypes.c_int, ctypes.c_int,
                                         ctypes.c_int, i64, ctypes.c_int, ctypes.POINTER(ctypes.c_float), vp]),
-    "gpk_test_tune": (ctypes.c_int, [ctypes.c_int, ctypes.c_int]),
     "gpk_test_overlap": (ctypes.c_int, [ctypes.c_int]),
     "gpk_test_position_lock": (ctypes.c_int, [ctypes.c_int]),
     "gpk_profile": (ctypes.c_int, [ctypes.c_int]),
     "gpk_profile_read": (ctypes.c_int, [c_double_p, ctypes.POINTER(i64), ctypes.POINTER(i64), c_double_p]),
-    "gpk_microbench": (ctypes.c_int, [ctypes.c_int, i64, c_double_p]),
     "gpk_microbench_i8": (ctypes.c_int, [i64, ctypes.c_double, c_double_p]),
 }
 

@@ -68,8 +68,12 @@ def test_library_is_sm100a_with_dmma(native):
     # ONE route: the CRT kernels (256x256 pair tiles + reconstruction pass); the round-1 variants are gone
     for kernel in ("oz_crt_planes_kernel", "oz_crt_reconstruct_kernel", "oz_residue_rows_kernel"):
         assert kernel in sass, kernel
-    for kernel in ("oz_crt_pair_kernel", "oz_gemm_pair_kernel", "oz_slice_rows_kernel"):
+    for kernel in ("oz_crt_pair_kernel", "oz_gemm_pair_kernel", "oz_slice_rows_kernel", "mb_dmma_kernel",
+                   "mb_dfma_kernel"):
         assert kernel not in sass, kernel
+    # one reconstruction kernel per epilogue (store, row sums) and group of 4 moduli (8..18 moduli: 2..5 groups)
+    functions = set(re.findall(r"Function : (\S+)", sass))
+    assert len([f for f in functions if "oz_crt_reconstruct_kernel" in f]) == 8
 
 
 def test_library_reads_no_environment_variables(native):

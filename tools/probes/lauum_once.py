@@ -1,4 +1,4 @@
-"""One K^-1 = X^T X shaped product (for ncu): python tools/probes/lauum_once.py [n] [position_lock] [group_m]"""
+"""One K^-1 = X^T X shaped product (for ncu): python tools/probes/lauum_once.py [n] [position_lock]"""
 import ctypes, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, os.path.join(ROOT, "scikit-gpuppy_b200"))
@@ -7,7 +7,6 @@ from skgpuppy import _native as nat
 lib = nat.load()
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 32768
 lib.gpk_test_position_lock(int(sys.argv[2]) if len(sys.argv) > 2 else 2)
-lib.gpk_test_tune(int(sys.argv[3]) if len(sys.argv) > 3 else 4, 1)
 dev = torch.device("cuda:0")
 g = torch.Generator(device=dev); g.manual_seed(0)
 X = torch.randn(n, n, dtype=torch.float64, device=dev, generator=g).tril_()
