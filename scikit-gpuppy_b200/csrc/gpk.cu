@@ -5,6 +5,7 @@
 
 #include <climits>
 #include <new>
+#include <type_traits>
 #include <vector>
 
 #include "dgemm_dmma.cuh"
@@ -27,7 +28,7 @@ struct Handle {
   double *X = nullptr, *W = nullptr;
   bool own_X = false, own_W = false;
   double *x = nullptr, *xT = nullptr, *t = nullptr, *y = nullptr, *alpha = nullptr, *dL = nullptr;
-  double* scal = nullptr;  // device scalars [8]
+  double* scal = nullptr;  // device scalars [3] of nll_scalars_kernel
   int* info = nullptr;
   double* part = nullptr; size_t part_elems = 0;      // partial-sum workspace
   double* G = nullptr; size_t G_elems = 0;            // per-batch query workspace rows x npad
@@ -63,7 +64,7 @@ struct Handle {
   bool ovl_on = false;
   // gradient prefetch (gpk_nll_grad with want_grad = 2): K^-1 and the trace sums are queued behind the factorisation
   // and land in pinned host memory; the gradient call at the same theta only waits for them
-  double* raw_pinned = nullptr;           // [3 * MAX_D + 8]
+  double* raw_pinned = nullptr;           // [TRACE_SUMS]
   bool grad_pending = false;
 };
 
@@ -121,6 +122,16 @@ static int ensure_overlap(Handle* h) {
 }
 
 static int theta_len(int kind, int d) { return kind == KIND_PERIODIC ? 2 + 3 * d : 2 + d; }
+
+// noise mode of the covariance tiles (periodic_tile_kernel): the periodic family adds vt wherever two points coincide,
+// the Gaussian family on the diagonal of the training K only
+static int noise_mode(int kind, bool training) { return kind == KIND_PERIODIC ? 2 : training ? 1 : 0; }
+
+// n/2 log(2 pi) + 1/2 log det K + 1/2 t^T K^-1 t of the cached factorisation (Covariance.py:211)
+static double nll_of(const Handle* h) {
+  const double two_pi = 6.283185307179586476925286766559;
+  return 0.5 * h->n * log(two_pi) + 0.5 * h->logdet + 0.5 * h->quad;
+}
 
 static int set_hyper(SEHyper& h, const double* theta, int d, int kind = KIND_SE) {
   if (d < 1 || d > MAX_D || (kind == KIND_PERIODIC && d > PER_MAX_D)) {
@@ -209,6 +220,23 @@ static int solve_one(Handle* h, const double* b_pad, double* y, double* out) {
   return 0;
 }
 
+// Pass width of the gradient-trace and exact-pair kernels: the dimensions of one pass are padded to DP, so the
+// per-thread accumulators are register arrays; the SE trace takes ceil(d / 32) passes beyond d = 32.
+static int pass_dim(int d) { return d <= 4 ? 4 : d <= 8 ? 8 : d <= 16 ? 16 : 32; }
+
+// f(std::integral_constant<int, pass_dim(d)>()), with only the widths up to MAX_DP instantiated
+template <int MAX_DP, int DP = 4, class F>
+static int dispatch_pass_dim(int d, F&& f) {
+  if constexpr (DP < MAX_DP) {
+    if (pass_dim(d) > DP) return dispatch_pass_dim<MAX_DP, 2 * DP>(d, f);
+  }
+  return f(std::integral_constant<int, DP>());
+}
+
+// doubles of the trace-sum vector (trace_enqueue): SE ceil(d / 32) passes of 33 + 2, periodic 3 * 16 + 2
+constexpr int TRACE_SUMS = (MAX_D + 31) / 32 * 33 + 2;
+static_assert(3 * PER_MAX_D + 2 <= TRACE_SUMS, "periodic trace sums exceed the trace-sum vector");
+
 template <int DP>
 static int launch_trace(Handle* h, int d0, int trb, int tre, double* partial) {
   const int nt = h->npad / TILE;
@@ -222,87 +250,94 @@ static int launch_trace(Handle* h, int d0, int trb, int tre, double* partial) {
   return 0;
 }
 
-// raw[0] = sum M Knl ; raw[1+k] = sum M Knl diff_k^2 over tile rows [trb, tre);
-// raw[d+1] = sum of diag(K^-1) and raw[d+2] = sum of alpha^2 over the same rows
-// async_dst != nullptr (Gaussian family only): nothing is synchronised, the sums go to that pinned buffer (trace_unpack)
-static int trace_sums(Handle* h, int trb, int tre, double* raw_host, double* async_dst = nullptr) {
-  const int d = h->d;
-  const int nt = h->npad / TILE;
-  for (int k = 0; k <= (h->kind == KIND_PERIODIC ? 3 * d + 2 : d + 2); ++k) raw_host[k] = 0.0;
+// Queue the trace sums of tile rows [trb, tre) of K^-1 and one copy of them to the host buffer dst (TRACE_SUMS doubles),
+// without synchronising. An empty range launches nothing and leaves dst alone. The device vector at the tail of h->part
+// has the layout dst receives, which only trace_unpack reads:
+//   SE, per pass p of DP dimensions: [p (DP + 1)] = sum M Knl, then sum M Knl diff_k^2 for k = p DP + j, j < DP;
+//       after the passes the sums of diag(K^-1) and of alpha^2 over the rows of the range
+//   periodic: the 3 DP + 2 column sums of periodic_trace_kernel<DP>
+static int trace_enqueue(Handle* h, int trb, int tre, double* dst) {
   if (tre <= trb) return 0;
-  if (h->kind != KIND_PERIODIC) {
-    const int r0 = trb * TILE, r1 = (tre * TILE < h->n) ? tre * TILE : h->n;
-    diag_sum_kernel<<<1, 256, 0, h->st>>>(h->W, h->npad, h->alpha, r0, r1, h->scal + 4);
-    GPK_LAUNCH_OK();
-    GPK_CUDA_OK(cudaMemcpyAsync(async_dst ? async_dst : raw_host + d + 1, h->scal + 4, 2 * sizeof(double),
-                                cudaMemcpyDeviceToHost, h->st));
-  }
-  if (h->kind == KIND_PERIODIC) {
-    // raw_host: [0] = sum M K, [1..d] diff^2 sums, [1+d..2d] diff sin cos sums, [1+2d..3d] sin^2 sums,
-    // then the sum of M over coincident pairs (the noise derivative) at [3d+1]; [3d+2] unused
-    const int DPp = d <= 4 ? 4 : d <= 8 ? 8 : 16;
-    const int nc = 3 * DPp + 2;
-    const long nsl = (long)nt * (tre - trb);
-    GPK_TRY(ensure(&h->part, &h->part_elems, (size_t)nsl * nc + nc));
-    double* psums = h->part + (size_t)nsl * nc;
-    dim3 pgrid(nt, tre - trb);
-    if (DPp == 4) periodic_trace_kernel<4><<<pgrid, 256, 0, h->st>>>(h->W, h->npad, h->alpha, h->x, h->n, d, h->hyp, trb, h->part);
-    else if (DPp == 8) periodic_trace_kernel<8><<<pgrid, 256, 0, h->st>>>(h->W, h->npad, h->alpha, h->x, h->n, d, h->hyp, trb, h->part);
-    else periodic_trace_kernel<16><<<pgrid, 256, 0, h->st>>>(h->W, h->npad, h->alpha, h->x, h->n, d, h->hyp, trb, h->part);
-    GPK_LAUNCH_OK();
-    col_sum_kernel<<<nc, 256, 0, h->st>>>(h->part, nsl, nc, psums);
-    GPK_LAUNCH_OK();
-    double ph[50];
-    GPK_CUDA_OK(cudaMemcpyAsync(ph, psums, nc * sizeof(double), cudaMemcpyDeviceToHost, h->st));
-    GPK_CUDA_OK(cudaStreamSynchronize(h->st));
-    raw_host[0] = ph[0];
-    for (int k = 0; k < d; ++k) {
-      raw_host[1 + k] = ph[1 + k];
-      raw_host[1 + d + k] = ph[1 + DPp + k];
-      raw_host[1 + 2 * d + k] = ph[1 + 2 * DPp + k];
-    }
-    raw_host[3 * d + 1] = ph[3 * DPp + 1];
-    raw_host[3 * d + 2] = 0.0;
-    return 0;
-  }
-  int DP = d <= 4 ? 4 : d <= 8 ? 8 : d <= 16 ? 16 : 32;
+  const int d = h->d, nt = h->npad / TILE;
   const long nslots = (long)nt * (tre - trb);
-  const int nchunks = (d + DP - 1) / DP;
-  GPK_TRY(ensure(&h->part, &h->part_elems, (size_t)nslots * (DP + 1) + (size_t)nchunks * (DP + 1)));
-  double* sums = h->part + (size_t)nslots * (DP + 1);
-  double host[2 * 33];
-  for (int d0 = 0, ch = 0; d0 < d; d0 += DP, ++ch) {
-    switch (DP) {
-      case 4: GPK_TRY(launch_trace<4>(h, d0, trb, tre, h->part)); break;
-      case 8: GPK_TRY(launch_trace<8>(h, d0, trb, tre, h->part)); break;
-      case 16: GPK_TRY(launch_trace<16>(h, d0, trb, tre, h->part)); break;
-      default: GPK_TRY(launch_trace<32>(h, d0, trb, tre, h->part)); break;
-    }
-    col_sum_kernel<<<DP + 1, 256, 0, h->st>>>(h->part, nslots, DP + 1, sums + ch * (DP + 1));
-    GPK_LAUNCH_OK();
-    double* dst = async_dst ? async_dst + 4 + ch * (DP + 1) : host + ch * 33;
-    GPK_CUDA_OK(cudaMemcpyAsync(dst, sums + ch * (DP + 1), (DP + 1) * sizeof(double), cudaMemcpyDeviceToHost, h->st));
+  double* sums = nullptr;
+  int nsums = 0;
+  if (h->kind == KIND_PERIODIC) {
+    GPK_TRY(dispatch_pass_dim<16>(d, [&](auto dp) {
+      constexpr int DP = decltype(dp)::value;
+      nsums = 3 * DP + 2;
+      GPK_TRY(ensure(&h->part, &h->part_elems, (size_t)nslots * nsums + nsums));
+      sums = h->part + (size_t)nslots * nsums;
+      periodic_trace_kernel<DP><<<dim3(nt, tre - trb), 256, 0, h->st>>>(h->W, h->npad, h->alpha, h->x, h->n, d, h->hyp,
+                                                                        trb, h->part);
+      GPK_LAUNCH_OK();
+      col_sum_kernel<<<nsums, 256, 0, h->st>>>(h->part, nslots, nsums, sums);
+      GPK_LAUNCH_OK();
+      return 0;
+    }));
+  } else {
+    GPK_TRY(dispatch_pass_dim<32>(d, [&](auto dp) {
+      constexpr int DP = decltype(dp)::value;
+      const int npass = (d + DP - 1) / DP;
+      nsums = npass * (DP + 1) + 2;
+      GPK_TRY(ensure(&h->part, &h->part_elems, (size_t)nslots * (DP + 1) + nsums));
+      sums = h->part + (size_t)nslots * (DP + 1);
+      const int r0 = trb * TILE, r1 = (tre * TILE < h->n) ? tre * TILE : h->n;
+      diag_sum_kernel<<<1, 256, 0, h->st>>>(h->W, h->npad, h->alpha, r0, r1, sums + npass * (DP + 1));
+      GPK_LAUNCH_OK();
+      for (int p = 0; p < npass; ++p) {
+        GPK_TRY(launch_trace<DP>(h, p * DP, trb, tre, h->part));
+        col_sum_kernel<<<DP + 1, 256, 0, h->st>>>(h->part, nslots, DP + 1, sums + p * (DP + 1));
+        GPK_LAUNCH_OK();
+      }
+      return 0;
+    }));
   }
-  if (async_dst) return 0;                      // trace_unpack reads the pinned buffer after the caller's sync
-  GPK_CUDA_OK(cudaStreamSynchronize(h->st));
-  for (int d0 = 0, ch = 0; d0 < d; d0 += DP, ++ch) {
-    if (d0 == 0) raw_host[0] = host[0];
-    for (int k = 0; k < DP && d0 + k < d; ++k) raw_host[1 + d0 + k] = host[ch * 33 + 1 + k];
-  }
+  GPK_CUDA_OK(cudaMemcpyAsync(dst, sums, nsums * sizeof(double), cudaMemcpyDeviceToHost, h->st));
   return 0;
 }
 
-// pinned layout of the asynchronous variant: [0..1] diag sums, [4 + ch (DP + 1) ...] chunk sums
-static void trace_unpack(const Handle* h, const double* pinned, double* raw_host) {
-  const int d = h->d;
-  const int DP = d <= 4 ? 4 : d <= 8 ? 8 : d <= 16 ? 16 : 32;
-  raw_host[d + 1] = pinned[0];
-  raw_host[d + 2] = pinned[1];
-  for (int d0 = 0, ch = 0; d0 < d; d0 += DP, ++ch) {
-    const double* src = pinned + 4 + ch * (DP + 1);
-    if (d0 == 0) raw_host[0] = src[0];
-    for (int k = 0; k < DP && d0 + k < d; ++k) raw_host[1 + d0 + k] = src[1 + k];
+// raw sums from the trace-sum vector of trace_enqueue:
+//   SE (d + 3): [0] = sum M Knl, [1 + k] = sum M Knl diff_k^2, [d + 1] = sum of diag(K^-1), [d + 2] = sum of alpha^2
+//   periodic (3 d + 3): [0] = sum M K, [1 + k] diff^2 sums, [1 + d + k] diff sin cos sums, [1 + 2d + k] sin^2 sums,
+//   [3d + 1] = sum of M over coincident pairs (the noise derivative), [3d + 2] = 0
+// Every SE pass sums M Knl again; the first pass's sum is the one used.
+static void trace_unpack(const Handle* h, const double* src, double* raw) {
+  const int d = h->d, DP = pass_dim(d);
+  raw[0] = src[0];
+  if (h->kind == KIND_PERIODIC) {
+    for (int k = 0; k < d; ++k) {
+      raw[1 + k] = src[1 + k];
+      raw[1 + d + k] = src[1 + DP + k];
+      raw[1 + 2 * d + k] = src[1 + 2 * DP + k];
+    }
+    raw[3 * d + 1] = src[3 * DP + 1];
+    raw[3 * d + 2] = 0.0;
+    return;
   }
+  for (int k = 0; k < d; ++k) raw[1 + k] = src[k / DP * (DP + 1) + 1 + k % DP];
+  const double* diag = src + (d + DP - 1) / DP * (DP + 1);
+  raw[d + 1] = diag[0];
+  raw[d + 2] = diag[1];
+}
+
+// the gradient from the raw trace sums of the whole K^-1 (trace_unpack)
+static void grad_from_raw(const Handle* h, const double* raw, double* grad) {
+  const int d = h->d;
+  grad[0] = 0.5 * raw[0];
+  if (h->kind == KIND_PERIODIC) {
+    // dK/dlog w_k = -1/2 w_k diff^2 K ; dK/dlog p_k = pi w2_k/p_k diff sin cos K ; dK/dlog w2_k = -1/2 w2_k sin^2 K
+    // (reference Covariance.py:420-433); the noise derivative is vt wherever two points coincide (:412-413)
+    grad[1] = 0.5 * h->hyp.vt * raw[3 * d + 1];
+    for (int k = 0; k < d; ++k) {
+      grad[2 + k] = -0.25 * h->hyp.w[k] * raw[1 + k];
+      grad[2 + d + k] = 0.5 * h->hyp.pf[k] * h->hyp.w2[k] * raw[1 + d + k];
+      grad[2 + 2 * d + k] = -0.25 * h->hyp.w2[k] * raw[1 + 2 * d + k];
+    }
+    return;
+  }
+  grad[1] = 0.5 * h->hyp.vt * (raw[d + 1] - raw[d + 2]);
+  for (int k = 0; k < d; ++k) grad[2 + k] = -0.25 * h->hyp.w[k] * raw[1 + k];
 }
 
 static int ensure_route(Handle* h);
@@ -487,7 +522,7 @@ static int create_fill(Handle* h, int64_t n, int64_t d, double* Xbuf, double* Wb
   GPK_CUDA_OK(cudaMalloc((void**)&h->y, np * sizeof(double)));
   GPK_CUDA_OK(cudaMalloc((void**)&h->alpha, np * sizeof(double)));
   GPK_CUDA_OK(cudaMalloc((void**)&h->dL, np * sizeof(double)));
-  GPK_CUDA_OK(cudaMalloc((void**)&h->scal, 8 * sizeof(double)));
+  GPK_CUDA_OK(cudaMalloc((void**)&h->scal, 3 * sizeof(double)));
   GPK_CUDA_OK(cudaMalloc((void**)&h->info, sizeof(int)));
   GPK_CUDA_OK(cudaMemset(h->t, 0, np * sizeof(double)));
   GPK_CUDA_OK(cudaMemset(h->alpha, 0, np * sizeof(double)));
@@ -698,8 +733,8 @@ int gpk_factorize(gpk_handle h, const double* theta, int want_inverse) {
     GPK_TRY(ensure_route(hh));
     const int n = hh->n, npad = hh->npad;
     // K (lower tiles) -> W
-    GPK_TRY(launch_se_tiles(hh->x, n, hh->x, n, hh->d, hh->hyp, hh->W, npad, npad, npad,
-                            hh->kind == KIND_PERIODIC ? 2 : 1, 1, 1, hh->st));
+    GPK_TRY(launch_se_tiles(hh->x, n, hh->x, n, hh->d, hh->hyp, hh->W, npad, npad, npad, noise_mode(hh->kind, true), 1,
+                            1, hh->st));
     const int rc = factorize_W(hh);
     if (rc != 0) return rc;
     memcpy(hh->theta, theta, sizeof(double) * theta_len(hh->kind, hh->d));
@@ -740,8 +775,7 @@ int gpk_factorize_matrix(gpk_handle h, const double* K_dev, int64_t ldk, int wan
 int gpk_nll_matrix(gpk_handle h, double* nll) {
   H_OR_FAIL(h);
   if (!hh->factored) { snprintf(g_err, sizeof(g_err), "not factored"); return -2; }
-  const double two_pi = 6.283185307179586476925286766559;
-  *nll = 0.5 * hh->n * log(two_pi) + 0.5 * hh->logdet + 0.5 * hh->quad;
+  *nll = nll_of(hh);
   return 0;
 }
 
@@ -759,7 +793,11 @@ int gpk_grad_trace_partial(gpk_handle h, int64_t trb, int64_t tre, double* out) 
   const int nt = hh->npad / TILE;
   if (trb < 0) trb = 0;
   if (tre > nt) tre = nt;
-  return trace_sums(hh, (int)trb, (int)tre, out);
+  double sums[TRACE_SUMS] = {};   // stays zero for an empty range
+  GPK_TRY(trace_enqueue(hh, (int)trb, (int)tre, sums));
+  GPK_CUDA_OK(cudaStreamSynchronize(hh->st));
+  trace_unpack(hh, sums, out);
+  return 0;
 }
 
 int gpk_nll_grad(gpk_handle h, const double* theta, double* nll, double* grad, int want_grad) {
@@ -772,42 +810,23 @@ int gpk_nll_grad(gpk_handle h, const double* theta, double* nll, double* grad, i
   }
   int rc = gpk_factorize(h, theta, want_grad == 1);
   if (rc != 0) return rc;
-  const double two_pi = 6.283185307179586476925286766559;
-  if (nll) *nll = 0.5 * hh->n * log(two_pi) + 0.5 * hh->logdet + 0.5 * hh->quad;
+  if (nll) *nll = nll_of(hh);
   if (prefetch && !hh->grad_pending) {
     // the caller announced that the gradient at this theta follows: queue K^-1 = X^T X and the trace sums now, so the
     // device keeps working while the host returns the likelihood
-    if (!hh->raw_pinned) GPK_CUDA_OK(cudaMallocHost((void**)&hh->raw_pinned, (3 * MAX_D + 8) * sizeof(double)));
+    if (!hh->raw_pinned) GPK_CUDA_OK(cudaMallocHost((void**)&hh->raw_pinned, TRACE_SUMS * sizeof(double)));
     GPK_TRY(do_lauum(hh));
-    double unused[3 * MAX_D + 3];
-    GPK_TRY(trace_sums(hh, 0, hh->npad / TILE, unused, hh->raw_pinned));
+    GPK_TRY(trace_enqueue(hh, 0, hh->npad / TILE, hh->raw_pinned));
     hh->grad_pending = true;
     return 0;
   }
   if (want_grad == 1 && grad) {
-    double raw[3 * MAX_D + 3];
-    if (hh->grad_pending) {
-      GPK_CUDA_OK(cudaStreamSynchronize(hh->st));
-      trace_unpack(hh, hh->raw_pinned, raw);
-      hh->grad_pending = false;
-    } else {
-      GPK_TRY(trace_sums(hh, 0, hh->npad / TILE, raw));
-    }
-    const int d = hh->d;
-    grad[0] = 0.5 * raw[0];
-    if (hh->kind == KIND_PERIODIC) {
-      // dK/dlog w_k = -1/2 w_k diff^2 K ; dK/dlog p_k = pi w2_k/p_k diff sin cos K ; dK/dlog w2_k = -1/2 w2_k sin^2 K
-      // (reference Covariance.py:420-433); the noise derivative is vt wherever two points coincide (:412-413)
-      grad[1] = 0.5 * hh->hyp.vt * raw[3 * d + 1];
-      for (int k = 0; k < d; ++k) {
-        grad[2 + k] = -0.25 * hh->hyp.w[k] * raw[1 + k];
-        grad[2 + d + k] = 0.5 * hh->hyp.pf[k] * hh->hyp.w2[k] * raw[1 + d + k];
-        grad[2 + 2 * d + k] = -0.25 * hh->hyp.w2[k] * raw[1 + 2 * d + k];
-      }
-      return 0;
-    }
-    grad[1] = 0.5 * hh->hyp.vt * (raw[hh->d + 1] - raw[hh->d + 2]);
-    for (int k = 0; k < hh->d; ++k) grad[2 + k] = -0.25 * hh->hyp.w[k] * raw[1 + k];
+    double sums[TRACE_SUMS], raw[3 * MAX_D + 3];
+    if (!hh->grad_pending) GPK_TRY(trace_enqueue(hh, 0, hh->npad / TILE, sums));
+    GPK_CUDA_OK(cudaStreamSynchronize(hh->st));
+    trace_unpack(hh, hh->grad_pending ? hh->raw_pinned : sums, raw);
+    hh->grad_pending = false;
+    grad_from_raw(hh, raw, grad);
   }
   return 0;
 }
@@ -837,6 +856,51 @@ int gpk_inverse(gpk_handle h, double* Kinv_out, int64_t ldo) {
   dim3 grid((n + 31) / 32, (n + 31) / 32);
   symmetrize_out_kernel<<<grid, 256, 0, hh->st>>>(hh->W, hh->npad, n, Kinv_out, ldo);
   GPK_LAUNCH_OK();
+  return 0;
+}
+
+// G[q][i] = Ks[q][i] for q < m, i < n; zero in the padding
+__global__ void __launch_bounds__(256) load_rows_kernel(const double* __restrict__ Ks, long ldk, int m, int n,
+                                                        double* __restrict__ G, long ldg, int npad) {
+  const int i = blockIdx.x * 256 + threadIdx.x;
+  const int q = blockIdx.y;
+  if (i >= npad) return;
+  G[(long)q * ldg + i] = (q < m && i < n) ? Ks[(long)q * ldk + i] : 0.0;
+}
+
+// The query batches of gpk_predict, gpk_predict_cross and the K alpha of gpk_solve_residual. Row q of G is the
+// covariance k(xq_q, x_i) from the family's tile kernel, or the caller's row Ks[q] when xq is null;
+// mean[q] = G_q . alpha (+ meant). With var: var[q] = prior[q] - |X G_q|^2, and v + vt in place of a null prior.
+static int query_batches(Handle* h, const double* xq, const double* Ks, long ldk, long m, double meant, double* mean,
+                         double* var, const double* prior) {
+  const int npad = h->npad, n = h->n, d = h->d, nbi = npad / TILE;
+  const long rows_max = batch_rows_for(h, m);
+  GPK_TRY(ensure_query_ws(h, rows_max));
+  for (long q0 = 0; q0 < m; q0 += rows_max) {
+    const long mb = (m - q0) < rows_max ? m - q0 : rows_max;
+    const long rows = round_up_l(mb, TILE);   // G zero padded to rows x npad
+    if (xq) {
+      GPK_TRY(launch_se_tiles(xq + q0 * d, (int)mb, h->x, n, d, h->hyp, h->G, npad, (int)rows, npad,
+                              noise_mode(h->kind, false), 0, 0, h->st));
+    } else {
+      load_rows_kernel<<<dim3((npad + 255) / 256, (unsigned)rows), 256, 0, h->st>>>(Ks + q0 * ldk, ldk, (int)mb, n,
+                                                                                    h->G, npad, npad);
+      GPK_LAUNCH_OK();
+    }
+    rows_dot_kernel<<<(unsigned)((mb + 7) / 8), 256, 0, h->st>>>(h->G, npad, (int)mb, npad, h->alpha, mean + q0);
+    GPK_LAUNCH_OK();
+    if (meant != 0.0) {
+      add_scalar_kernel<<<(unsigned)((mb + 255) / 256), 256, 0, h->st>>>(mean + q0, (int)mb, meant);
+      GPK_LAUNCH_OK();
+    }
+    if (var) {
+      GPK_TRY(quad_forms(h, rows));
+      predict_var_kernel<<<(unsigned)((mb + 255) / 256), 256, 0, h->st>>>(h->colsq, rows, nbi, (int)mb,
+                                                                          prior ? prior + q0 : nullptr,
+                                                                          h->hyp.v + h->hyp.vt, var + q0);
+      GPK_LAUNCH_OK();
+    }
+  }
   return 0;
 }
 
@@ -870,21 +934,13 @@ __global__ void __launch_bounds__(256) residual_max_kernel(const double* __restr
 int gpk_solve_residual(gpk_handle h, double* out_host) {
   H_OR_FAIL(h);
   if (!hh->factored || hh->matrix_state) { snprintf(g_err, sizeof(g_err), "not factored from theta"); return -2; }
-  const int npad = hh->npad, n = hh->n, d = hh->d;
+  const int n = hh->n;
   // K alpha with K regenerated tile row by tile row in the query workspace (K itself was consumed by the factorisation)
-  const long rows_max = batch_rows_for(hh, n);
-  GPK_TRY(ensure_query_ws(hh, rows_max));
-  GPK_TRY(ensure(&hh->part, &hh->part_elems, (size_t)npad + 8));
+  GPK_TRY(ensure(&hh->part, &hh->part_elems, (size_t)hh->npad + 8));
   double* Ka = hh->part;
-  unsigned long long* mx = reinterpret_cast<unsigned long long*>(hh->part + npad);
+  unsigned long long* mx = reinterpret_cast<unsigned long long*>(hh->part + hh->npad);
   GPK_CUDA_OK(cudaMemsetAsync(mx, 0, 3 * sizeof(unsigned long long), hh->st));
-  for (long r0 = 0; r0 < n; r0 += rows_max) {
-    const long mb = (n - r0) < rows_max ? (long)(n - r0) : rows_max;
-    GPK_TRY(launch_se_tiles(hh->x + r0 * d, (int)mb, hh->x, n, d, hh->hyp, hh->G, npad, (int)mb, npad,
-                            hh->kind == KIND_PERIODIC ? 2 : 0, 0, 0, hh->st));
-    rows_dot_kernel<<<(unsigned)((mb + 7) / 8), 256, 0, hh->st>>>(hh->G, npad, (int)mb, npad, hh->alpha, Ka + r0);
-    GPK_LAUNCH_OK();
-  }
+  GPK_TRY(query_batches(hh, hh->x, nullptr, 0, n, 0.0, Ka, nullptr, nullptr));
   if (hh->kind != KIND_PERIODIC) {
     // the Gaussian family adds vt on the diagonal only (Covariance.py:461-464): (K alpha)_i += vt alpha_i
     axpy_kernel<<<(n + 255) / 256, 256, 0, hh->st>>>(Ka, hh->alpha, n, hh->hyp.vt);
@@ -924,49 +980,7 @@ int gpk_predict(gpk_handle h, const double* xs, int64_t m, double meant, double*
   H_OR_FAIL(h);
   if (!hh->factored || hh->matrix_state) { snprintf(g_err, sizeof(g_err), "not factored from theta"); return -2; }
   if (m <= 0) return 0;
-  const int npad = hh->npad, n = hh->n, d = hh->d;
-  const long rows_max = batch_rows_for(hh, m);
-  GPK_TRY(ensure_query_ws(hh, rows_max));
-  const int nbi = npad / TILE;
-  for (int64_t q0 = 0; q0 < m; q0 += rows_max) {
-    const long mb = (m - q0) < rows_max ? (long)(m - q0) : rows_max;
-    const long rows = round_up_l(mb, TILE);
-    // G[q][i] = k(xs_q, x_i), zero padded to rows x npad
-    GPK_TRY(launch_se_tiles(xs + q0 * d, (int)mb, hh->x, n, d, hh->hyp, hh->G, npad, (int)rows, npad,
-                            hh->kind == KIND_PERIODIC ? 2 : 0, 0, 0, hh->st));
-    rows_dot_kernel<<<(unsigned)((mb + 7) / 8), 256, 0, hh->st>>>(hh->G, npad, (int)mb, npad, hh->alpha, mean + q0);
-    GPK_LAUNCH_OK();
-    if (meant != 0.0) {
-      add_scalar_kernel<<<(unsigned)((mb + 255) / 256), 256, 0, hh->st>>>(mean + q0, (int)mb, meant);
-      GPK_LAUNCH_OK();
-    }
-    if (want_var) {
-      GPK_TRY(quad_forms(hh, rows));
-      predict_var_kernel<<<(unsigned)((mb + 255) / 256), 256, 0, hh->st>>>(hh->colsq, rows, nbi, (int)mb,
-                                                                            hh->hyp.v + hh->hyp.vt, var + q0);
-      GPK_LAUNCH_OK();
-    }
-  }
-  return 0;
-}
-
-// G[q][i] = Ks[q][i] for q < m, i < n; zero in the padding
-__global__ void __launch_bounds__(256) load_rows_kernel(const double* __restrict__ Ks, long ldk, int m, int n,
-                                                        double* __restrict__ G, long ldg, int npad) {
-  const int i = blockIdx.x * 256 + threadIdx.x;
-  const int q = blockIdx.y;
-  if (i >= npad) return;
-  G[(long)q * ldg + i] = (q < m && i < n) ? Ks[(long)q * ldk + i] : 0.0;
-}
-// var[q] = prior[q] - sum_b colsq[b][q]
-__global__ void __launch_bounds__(256) predict_var_prior_kernel(const double* __restrict__ colsq, long ldo, int nbi, int m,
-                                                                const double* __restrict__ prior,
-                                                                double* __restrict__ var) {
-  const int q = blockIdx.x * 256 + threadIdx.x;
-  if (q >= m) return;
-  double s = 0.0;
-  for (int b = 0; b < nbi; ++b) s += colsq[(long)b * ldo + q];
-  var[q] = prior[q] - s;
+  return query_batches(hh, xs, nullptr, 0, m, meant, mean, want_var ? var : nullptr, nullptr);
 }
 
 int gpk_predict_cross(gpk_handle h, const double* Ks, int64_t ldk, int64_t m, const double* prior, double meant,
@@ -974,31 +988,11 @@ int gpk_predict_cross(gpk_handle h, const double* Ks, int64_t ldk, int64_t m, co
   H_OR_FAIL(h);
   if (!hh->factored) { snprintf(g_err, sizeof(g_err), "not factored"); return -2; }
   if (m <= 0) return 0;
-  if (!Ks || ldk < hh->n) { snprintf(g_err, sizeof(g_err), "gpk_predict_cross: bad cross-covariance argument"); return -2; }
-  const int npad = hh->npad, n = hh->n;
-  const long rows_max = batch_rows_for(hh, m);
-  GPK_TRY(ensure_query_ws(hh, rows_max));
-  const int nbi = npad / TILE;
-  for (int64_t q0 = 0; q0 < m; q0 += rows_max) {
-    const long mb = (m - q0) < rows_max ? (long)(m - q0) : rows_max;
-    const long rows = round_up_l(mb, TILE);
-    dim3 lg((npad + 255) / 256, (unsigned)rows);
-    load_rows_kernel<<<lg, 256, 0, hh->st>>>(Ks + q0 * ldk, ldk, (int)mb, n, hh->G, npad, npad);
-    GPK_LAUNCH_OK();
-    rows_dot_kernel<<<(unsigned)((mb + 7) / 8), 256, 0, hh->st>>>(hh->G, npad, (int)mb, npad, hh->alpha, mean + q0);
-    GPK_LAUNCH_OK();
-    if (meant != 0.0) {
-      add_scalar_kernel<<<(unsigned)((mb + 255) / 256), 256, 0, hh->st>>>(mean + q0, (int)mb, meant);
-      GPK_LAUNCH_OK();
-    }
-    if (var) {
-      GPK_TRY(quad_forms(hh, rows));
-      predict_var_prior_kernel<<<(unsigned)((mb + 255) / 256), 256, 0, hh->st>>>(hh->colsq, rows, nbi, (int)mb,
-                                                                                  prior + q0, var + q0);
-      GPK_LAUNCH_OK();
-    }
+  if (!Ks || ldk < hh->n || (var && !prior)) {
+    snprintf(g_err, sizeof(g_err), "gpk_predict_cross: bad cross-covariance argument");
+    return -2;
   }
-  return 0;
+  return query_batches(hh, nullptr, Ks, ldk, m, meant, mean, var, prior);
 }
 
 static int propagate_impl(gpk_handle h, const double* U, const double* S, int64_t Q, int sigma_full, double meant,
@@ -1065,11 +1059,11 @@ int gpk_propagate_exact(gpk_handle h, const double* U, const double* Lam, const 
     exact_g_kernel<<<ggrid, 256, 0, hh->st>>>(a, hh->hyp, gq);
     GPK_LAUNCH_OK();
     dim3 grid(qb, nt);
-    if (d <= 4) exact_pair_kernel<4><<<grid, 256, 0, hh->st>>>(a, gq, hh->part);
-    else if (d <= 8) exact_pair_kernel<8><<<grid, 256, 0, hh->st>>>(a, gq, hh->part);
-    else if (d <= 16) exact_pair_kernel<16><<<grid, 256, 0, hh->st>>>(a, gq, hh->part);
-    else exact_pair_kernel<32><<<grid, 256, 0, hh->st>>>(a, gq, hh->part);
-    GPK_LAUNCH_OK();
+    GPK_TRY(dispatch_pass_dim<32>(d, [&](auto dp) {
+      exact_pair_kernel<decltype(dp)::value><<<grid, 256, 0, hh->st>>>(a, gq, hh->part);
+      GPK_LAUNCH_OK();
+      return 0;
+    }));
     exact_finalize_kernel<<<(qb + 255) / 256, 256, 0, hh->st>>>(hh->part, nt, mu, a.norms, qb, hh->hyp.v + hh->hyp.vt,
                                                                  meant, mean + q0, var + q0);
     GPK_LAUNCH_OK();

@@ -401,14 +401,15 @@ __global__ void __launch_bounds__(256) ga_finalize_kernel(const double* __restri
   if (rest_out) rest_out[q] = rest;
 }
 
-// var[q] = v + vt - sum_b colsq[b][q]
+// var[q] = prior[q] - sum_b colsq[b][q], or v + vt - sum_b colsq[b][q] without a prior vector
 __global__ void __launch_bounds__(256) predict_var_kernel(const double* __restrict__ colsq, long ldo, int nbi, int m,
-                                                          double vpvt, double* __restrict__ var) {
+                                                          const double* __restrict__ prior, double vpvt,
+                                                          double* __restrict__ var) {
   const int q = blockIdx.x * 256 + threadIdx.x;
   if (q >= m) return;
   double s = 0.0;
   for (int b = 0; b < nbi; ++b) s += colsq[(long)b * ldo + q];
-  var[q] = vpvt - s;
+  var[q] = (prior ? prior[q] : vpvt) - s;
 }
 
 __global__ void __launch_bounds__(256) add_scalar_kernel(double* __restrict__ y, int len, double a) {

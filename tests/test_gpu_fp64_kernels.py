@@ -9,7 +9,7 @@ the tolerances sit at the kernel's rounding: a sum is compared relative to the s
 observed ratio to the bound, so the margin is in the log (run with -s).
 
   A  leaf_blocked_kernel + the sub-2048 DMMA recursion (gpk_test_potrf_inv): X = L^-1, diag L, first bad pivot
-  B  grad_trace_kernel<4|8|16|32> (one and two passes), trace_sums / trace_unpack, periodic_trace_kernel<4|8|16>
+  B  grad_trace_kernel<4|8|16|32> (one and two passes), trace_enqueue / trace_unpack, periodic_trace_kernel<4|8|16>
   C  exact_pair_kernel<4|8|16|32> through UncertaintyPropagationExact
   D  non-positive-definite K through gpk_factorize_matrix on the DMMA and INT8 routes
 """
@@ -358,7 +358,7 @@ def test_se_trace_partial_vs_longdouble(gpk, n, d):
     ra = report("SE gradient n=%d d=%d: vs DenseArbiter at 1e-9" % (n, d),
                 float(np.max(np.abs(g.astype(LD) - ga)) / np.max(np.abs(ga)) / 1e-9))
     assert ra <= 1.0
-    # the prefetch path (want_grad = 2): same kernels, sums collected from the pinned chunk layout of trace_unpack
+    # the prefetch path (want_grad = 2): same kernels and sum layout, copied to the pinned buffer and unpacked later
     eng.nll_grad(theta + 1e-3, want_grad=False)
     eng.nll_grad(theta, want_grad=False, prefetch_grad=True)
     _, g2 = eng.nll_grad(theta, want_grad=True)
