@@ -142,6 +142,28 @@ int gpk_predict_cross(gpk_handle h, const double* Ks_dev, int64_t ldk, int64_t m
                       double* mean_dev, double* var_dev);
 
 /*
+ * Joint predictive covariance (the matrix the reference forms inside estimate_many, GaussianProcess.py:75-80):
+ * cov[a*ldc + b] = k(xa_a, xb_b) + noise - k(xa_a, x) K^-1 k(x, xb_b), with k(., x) = K* rows as in gpk_predict.
+ * xb_dev == NULL: B = A (mb is ignored). The output is ma x ma and exactly symmetric, and the noise term follows
+ * cov_matrix(A) of the family. xb_dev != NULL: the noise term follows cov_matrix_ij(A, B).
+ * Needs gpk_factorize (theta state), like gpk_predict. ma == 0 or mb == 0 does nothing.
+ * Workspace: the rows of V = X k(x, .) of both sets stay resident for the call (8 * m_pad * npad bytes per set, plus
+ * moduli * m_pad * npad bytes of their residues on the INT8 route) with a padded ma x mb output block and one query
+ * batch; if that does not fit the call returns -4 before any work is queued (byte counts in gpk_last_error()).
+ */
+int gpk_predict_cov(gpk_handle h, const double* xa_dev, int64_t ma, const double* xb_dev, int64_t mb,
+                    double* cov_dev, int64_t ldc);
+
+/*
+ * Same from caller-built cross covariances (covariance classes without device kernels; works after
+ * gpk_factorize or gpk_factorize_matrix): Ka is ma x n (lda), Kb is mb x n (ldb) or NULL for B = A,
+ * prior is the caller's ma x mb block k(A, B) including its noise (ldp). cov_dev may equal prior_dev.
+ */
+int gpk_predict_cov_cross(gpk_handle h, const double* Ka_dev, int64_t lda, int64_t ma,
+                          const double* Kb_dev, int64_t ldb, int64_t mb,
+                          const double* prior_dev, int64_t ldp, double* cov_dev, int64_t ldc);
+
+/*
  * Girard Gaussian approximation, batched over Q queries (UncertaintyPropagationApprox.propagate_GA,
  * UncertaintyPropagation2.pyx:266-299 with :208-257). U: Q x d means. S: Q x d (diagonal of Sigma_x) or,
  * with sigma_full, Q x d x d. Includes the equality-noise quirk of the scalar covariance (Covariance.py:451).

@@ -35,6 +35,8 @@ struct Handle {
   double* colsq = nullptr; size_t colsq_elems = 0;    // [nbi][rows]
   double* pairdot = nullptr;                          // [nbi][rows/2]
   double* dots = nullptr; size_t dots_elems = 0;      // [rows]
+  double* V = nullptr; size_t V_elems = 0;            // gpk_predict_cov: rows of V^T = G X^T of both query sets
+  double* C = nullptr; size_t C_elems = 0;            // gpk_predict_cov: padded output block
   long batch_rows = 0;                                // user cap on rows per batch (0 = default)
   SEHyper hyp;
   int kind = KIND_SE;                     // covariance family (gpk_set_kernel)
@@ -410,13 +412,22 @@ static int ensure_route(Handle* h) {
   return ensure_overlap(h);
 }
 
-// colsq/pairdot partials of V = X * G^T for `rows` rows of G (multiple of 128)
-static int quad_forms(Handle* h, long rows) {
+// residue planes of a rows x cols query product (INT8 route): 4 GiB at most, row panels beyond
+static int ensure_query_planes(Handle* h, long rows, long cols) {
+  size_t want_out = (size_t)h->oz.S * round_up_l(rows, 256) * round_up_l(cols, 256);
+  const size_t qcap = oz_out_cap_bytes(h) < ((size_t)4 << 30) ? oz_out_cap_bytes(h) : ((size_t)4 << 30);
+  if (want_out > qcap) want_out = qcap;
+  return h->ozq.ensure_out(want_out);
+}
+
+// V = X * G^T for `rows` rows of G (multiple of 128). Vt == nullptr: only its colsq/pairdot partials (predictive
+// variances, Girard quadratic forms); else V^T = G X^T itself, stored to Vt (rows x npad, leading dimension npad).
+static int quad_forms(Handle* h, long rows, double* Vt = nullptr) {
   GPK_TRY(ensure_route(h));
+  const int npad = h->npad;
   if (h->oz_on) {
     // INT8 tensor-core route: V^T = G X^T with the queries as rows, so each reconstruction warp sums its own row.
     // X is reduced once per factorisation (kept in the workspace), G once per batch.
-    const int npad = h->npad;
     if (!h->x_sliced) {
       h->oz.reset();
       h->xs = h->oz.alloc(npad, npad);
@@ -425,19 +436,21 @@ static int quad_forms(Handle* h, long rows) {
       h->x_sliced = true;
     }
     h->ozq.S = h->oz.S;
-    size_t want_out = (size_t)h->oz.S * round_up_l(rows, 256) * round_up_l((long)npad, 256);
-    const size_t qcap = oz_out_cap_bytes(h) < ((size_t)4 << 30) ? oz_out_cap_bytes(h) : ((size_t)4 << 30);
-    if (want_out > qcap) want_out = qcap;      // query batches: 4 GiB of planes, row panels beyond
-    if (h->ozq.ensure((size_t)h->oz.S * rows * npad, (size_t)rows, (size_t)rows) != 0 || h->ozq.ensure_out(want_out) != 0) {
+    if (h->ozq.ensure((size_t)h->oz.S * rows * npad, (size_t)rows, (size_t)rows) != 0 ||
+        ensure_query_planes(h, rows, npad) != 0) {
       snprintf(g_err, sizeof(g_err), "INT8 route: query workspace for %ld rows does not fit on the device", rows);
       return -4;
     }
     h->ozq.reset();
     oz::Operand g = h->ozq.alloc((int)rows, npad);
     GPK_TRY(oz::slice_operand(h->G, npad, 0, 0, g, h->ozq.mx, h->st));
+    if (Vt) return oz::gemm_sliced(g, h->xs, Vt, npad, 1.0, 0.0, K_UPTO_BJ, 0, h->st);
     return oz::gemm_sliced(g, h->xs, nullptr, 0, 1.0, 0.0, K_UPTO_BJ, 0, h->st, oz::OZ_EPI_ROWSQ, h->colsq, h->pairdot,
                            rows);
   }
+  if (Vt)   // the L21 = A21 X11^T form of the factorisation
+    return gemm_store_auto<LAY_KC, LAY_KC>(
+        gemm_args(h->G, npad, h->X, npad, Vt, npad, (int)rows, npad, npad, 1.0, 0.0, K_UPTO_BJ, 0), h->st);
   GemmArgs a = gemm_args(h->X, h->npad, h->G, h->npad, nullptr, 0, h->npad, (int)rows, h->npad, 1.0, 0.0, K_UPTO_BI, 0);
   a.colsq = h->colsq;
   a.pairdot = h->pairdot;
@@ -575,6 +588,8 @@ int gpk_destroy(gpk_handle h) {
   if (hh->G) cudaFree(hh->G);
   if (hh->colsq) cudaFree(hh->colsq);
   if (hh->dots) cudaFree(hh->dots);
+  if (hh->V) cudaFree(hh->V);
+  if (hh->C) cudaFree(hh->C);
   hh->oz.release();
   hh->ozq.release();
   release_overlap(hh);
@@ -869,10 +884,11 @@ __global__ void __launch_bounds__(256) load_rows_kernel(const double* __restrict
 }
 
 // The query batches of gpk_predict, gpk_predict_cross and the K alpha of gpk_solve_residual. Row q of G is the
-// covariance k(xq_q, x_i) from the family's tile kernel, or the caller's row Ks[q] when xq is null;
-// mean[q] = G_q . alpha (+ meant). With var: var[q] = prior[q] - |X G_q|^2, and v + vt in place of a null prior.
+// covariance k(xq_q, x_i) from the family's tile kernel, or the caller's row Ks[q] when xq is null.
+// With mean: mean[q] = G_q . alpha (+ meant). With var: var[q] = prior[q] - |X G_q|^2, and v + vt in place of a null
+// prior. With Vt (gpk_predict_cov): row q of Vt = (X G_q)^T, round_up(m, 128) rows of npad, zero beyond row m.
 static int query_batches(Handle* h, const double* xq, const double* Ks, long ldk, long m, double meant, double* mean,
-                         double* var, const double* prior) {
+                         double* var, const double* prior, double* Vt = nullptr) {
   const int npad = h->npad, n = h->n, d = h->d, nbi = npad / TILE;
   const long rows_max = batch_rows_for(h, m);
   GPK_TRY(ensure_query_ws(h, rows_max));
@@ -887,12 +903,15 @@ static int query_batches(Handle* h, const double* xq, const double* Ks, long ldk
                                                                                     h->G, npad, npad);
       GPK_LAUNCH_OK();
     }
-    rows_dot_kernel<<<(unsigned)((mb + 7) / 8), 256, 0, h->st>>>(h->G, npad, (int)mb, npad, h->alpha, mean + q0);
-    GPK_LAUNCH_OK();
-    if (meant != 0.0) {
-      add_scalar_kernel<<<(unsigned)((mb + 255) / 256), 256, 0, h->st>>>(mean + q0, (int)mb, meant);
+    if (mean) {
+      rows_dot_kernel<<<(unsigned)((mb + 7) / 8), 256, 0, h->st>>>(h->G, npad, (int)mb, npad, h->alpha, mean + q0);
       GPK_LAUNCH_OK();
+      if (meant != 0.0) {
+        add_scalar_kernel<<<(unsigned)((mb + 255) / 256), 256, 0, h->st>>>(mean + q0, (int)mb, meant);
+        GPK_LAUNCH_OK();
+      }
     }
+    if (Vt) GPK_TRY(quad_forms(h, rows, Vt + q0 * npad));
     if (var) {
       GPK_TRY(quad_forms(h, rows));
       predict_var_kernel<<<(unsigned)((mb + 255) / 256), 256, 0, h->st>>>(h->colsq, rows, nbi, (int)mb,
@@ -900,6 +919,72 @@ static int query_batches(Handle* h, const double* xq, const double* Ks, long ldk
                                                                           h->hyp.v + h->hyp.vt, var + q0);
       GPK_LAUNCH_OK();
     }
+  }
+  return 0;
+}
+
+// Joint predictive covariance Sigma(A, B) = prior(A, B) - V_A^T V_B, V_Q = X k(x, Q), for gpk_predict_cov and
+// gpk_predict_cov_cross. Rows of A / B come from the query points xa / xb through the family's tile kernel, or from the
+// caller's cross covariances Ka / Kb; prior is the caller's block (ldp), else k(A, B) with the family's noise rule.
+// xb and Kb both null: B = A, only the lower tiles are formed and mirrored on the way out, so the result is exactly
+// symmetric. V^T of both sets stays resident for the call and the product runs once over K = npad, on the route of
+// the factorisation; if its workspace does not fit, the call fails with -4 before any work is queued.
+static int predict_cov_impl(Handle* h, const double* xa, const double* Ka, long lda, long ma, const double* xb,
+                            const double* Kb, long ldb, long mb, const double* prior, long ldp, double* cov, long ldc) {
+  const bool sym = !xb && !Kb;
+  const long npad = h->npad;
+  const long ma_pad = round_up_l(ma, TILE), mb_pad = sym ? ma_pad : round_up_l(mb, TILE);
+  const long vrows = sym ? ma_pad : ma_pad + mb_pad;
+  GPK_TRY(ensure_route(h));
+  // every allocation of the call, before any of its work is queued: V, the output block, the query batch (G and its
+  // partials), and on the INT8 route the residues of V (which also hold those of G) and the planes of both products
+  const long mmax = ma_pad > mb_pad ? ma_pad : mb_pad;
+  const long rows_max = batch_rows_for(h, mmax);
+  const size_t res_bytes = h->oz_on ? (size_t)h->oz.S * vrows * npad : 0;
+  if (ensure(&h->V, &h->V_elems, (size_t)vrows * npad) != 0 || ensure(&h->C, &h->C_elems, (size_t)ma_pad * mb_pad) != 0 ||
+      ensure_query_ws(h, rows_max) != 0 ||
+      (h->oz_on && (h->ozq.ensure(res_bytes, (size_t)vrows, (size_t)mmax) != 0 ||
+                    ensure_query_planes(h, rows_max, npad) != 0 || ensure_query_planes(h, ma_pad, mb_pad) != 0))) {
+    cudaGetLastError();   // the failed allocation is reported here, not by the next call
+    snprintf(g_err, sizeof(g_err),
+             "predictive covariance %ld x %ld at n=%d: %.2f GB of V + %.2f GB of output block + %.2f GB of query batch "
+             "+ %.2f GB of V residues do not fit on the device",
+             ma, mb, h->n, 8.0 * vrows * npad / 1e9, 8.0 * ma_pad * mb_pad / 1e9, 8.0 * rows_max * npad / 1e9,
+             (double)res_bytes / 1e9);
+    return -4;
+  }
+  double* Va = h->V;
+  double* Vb = sym ? h->V : h->V + ma_pad * npad;
+  GPK_TRY(query_batches(h, xa, Ka, lda, ma, 0.0, nullptr, nullptr, nullptr, Va));
+  if (!sym) GPK_TRY(query_batches(h, xb, Kb, ldb, mb, 0.0, nullptr, nullptr, nullptr, Vb));
+  // the padding of the output block is never copied out: a caller's prior leaves it unset
+  if (prior) {
+    GPK_CUDA_OK(cudaMemcpy2DAsync(h->C, mb_pad * sizeof(double), prior, ldp * sizeof(double), mb * sizeof(double), ma,
+                                  cudaMemcpyDeviceToDevice, h->st));
+  } else {
+    GPK_TRY(launch_se_tiles(xa, (int)ma, sym ? xa : xb, (int)mb, h->d, h->hyp, h->C, mb_pad, (int)ma_pad, (int)mb_pad,
+                            noise_mode(h->kind, sym), 0, sym ? 1 : 0, h->st));
+  }
+  if (h->oz_on) {
+    // the residues of G are consumed by the V products queued above; the residues of V replace them
+    h->ozq.reset();
+    oz::Operand a = h->ozq.alloc((int)ma_pad, (int)npad);
+    oz::Operand b = sym ? a : h->ozq.alloc((int)mb_pad, (int)npad);
+    GPK_TRY(oz::slice_operand(Va, npad, 0, 0, a, h->ozq.mx, h->st));
+    if (!sym) GPK_TRY(oz::slice_operand(Vb, npad, 0, 0, b, h->ozq.mx, h->st));
+    GPK_TRY(oz::gemm_sliced(a, sym ? a : b, h->C, mb_pad, -1.0, 1.0, K_FULL, sym ? 1 : 0, h->st));
+  } else {
+    GPK_TRY((gemm_store_auto<LAY_KC, LAY_KC>(
+        gemm_args(Va, npad, Vb, npad, h->C, mb_pad, (int)ma_pad, (int)mb_pad, (int)npad, -1.0, 1.0, K_FULL, sym ? 1 : 0),
+        h->st)));
+  }
+  if (sym) {
+    dim3 grid((unsigned)((ma + 31) / 32), (unsigned)((ma + 31) / 32));
+    symmetrize_out_kernel<<<grid, 256, 0, h->st>>>(h->C, mb_pad, (int)ma, cov, ldc);
+    GPK_LAUNCH_OK();
+  } else {
+    GPK_CUDA_OK(cudaMemcpy2DAsync(cov, ldc * sizeof(double), h->C, mb_pad * sizeof(double), mb * sizeof(double), ma,
+                                  cudaMemcpyDeviceToDevice, h->st));
   }
   return 0;
 }
@@ -993,6 +1078,30 @@ int gpk_predict_cross(gpk_handle h, const double* Ks, int64_t ldk, int64_t m, co
     return -2;
   }
   return query_batches(hh, nullptr, Ks, ldk, m, meant, mean, var, prior);
+}
+
+int gpk_predict_cov(gpk_handle h, const double* xa, int64_t ma, const double* xb, int64_t mb, double* cov, int64_t ldc) {
+  H_OR_FAIL(h);
+  if (!hh->factored || hh->matrix_state) { snprintf(g_err, sizeof(g_err), "not factored from theta"); return -2; }
+  if (!xb) mb = ma;
+  if (ma < 0 || mb < 0) { snprintf(g_err, sizeof(g_err), "gpk_predict_cov: negative query count"); return -2; }
+  if (ma == 0 || mb == 0) return 0;
+  if (!xa || !cov || ldc < mb) { snprintf(g_err, sizeof(g_err), "gpk_predict_cov: bad query or output argument"); return -2; }
+  return predict_cov_impl(hh, xa, nullptr, 0, ma, xb, nullptr, 0, mb, nullptr, 0, cov, ldc);
+}
+
+int gpk_predict_cov_cross(gpk_handle h, const double* Ka, int64_t lda, int64_t ma, const double* Kb, int64_t ldb,
+                          int64_t mb, const double* prior, int64_t ldp, double* cov, int64_t ldc) {
+  H_OR_FAIL(h);
+  if (!hh->factored) { snprintf(g_err, sizeof(g_err), "not factored"); return -2; }
+  if (!Kb) mb = ma;
+  if (ma < 0 || mb < 0) { snprintf(g_err, sizeof(g_err), "gpk_predict_cov_cross: negative query count"); return -2; }
+  if (ma == 0 || mb == 0) return 0;
+  if (!Ka || lda < hh->n || (Kb && ldb < hh->n) || !prior || ldp < mb || !cov || ldc < mb) {
+    snprintf(g_err, sizeof(g_err), "gpk_predict_cov_cross: bad cross-covariance, prior or output argument");
+    return -2;
+  }
+  return predict_cov_impl(hh, nullptr, Ka, lda, ma, nullptr, Kb, ldb, mb, prior, ldp, cov, ldc);
 }
 
 static int propagate_impl(gpk_handle h, const double* U, const double* S, int64_t Q, int sigma_full, double meant,

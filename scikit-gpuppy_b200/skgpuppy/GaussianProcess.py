@@ -163,6 +163,55 @@ class GaussianProcess(object):
         """Same on device-resident queries; returns CUDA tensors."""
         return self._engine().predict_device(xs_dev, self.meant, want_var=want_var)
 
+    # -- joint predictive covariance (an addition: the matrix the reference forms inside estimate_many,
+    #    GaussianProcess.py:75-80, of which it returns only the diagonal) ------------------------------------------------
+    def _no_sparse(self, what):
+        if hasattr(self.cov, "_sparse_predict"):
+            raise NotImplementedError("%s: the low-rank predictive covariance of %s is not implemented"
+                                      % (what, type(self.cov).__name__))
+
+    def estimate_many_cov(self, x_stars):
+        """Means (m,) and the joint predictive covariance (m, m), noise included, at the rows of x_stars. The means are
+        those of estimate_many, the diagonal of the covariance its variances; the matrix is exactly symmetric."""
+        self._no_sparse("estimate_many_cov")
+        if np.size(x_stars) == 0:
+            return np.zeros(0), np.zeros((0, 0))
+        xs = self._queries(x_stars)
+        eng = self._engine()
+        if getattr(self.cov, "_KIND", None) is None:
+            kv = eng.to_device(np.asarray(self.cov.cov_matrix_ij(xs, self.x, self.theta_min), dtype=np.float64))
+            prior = eng.to_device(np.asarray(self.cov.cov_matrix(xs, self.theta_min), dtype=np.float64))
+            mean, _ = eng.predict_cross_device(kv, None, self.meant, want_var=False)
+            cov = eng.predict_cov_cross_device(kv, None, prior)
+        else:
+            mean, cov = self.estimate_many_cov_device(eng.to_device(xs))
+        return mean.cpu().numpy(), cov.cpu().numpy()
+
+    def estimate_many_cov_device(self, xs_dev):
+        """Same on device-resident queries (covariance classes with device kernels); returns CUDA tensors."""
+        self._no_sparse("estimate_many_cov_device")
+        eng = self._engine()
+        mean, _ = eng.predict_device(xs_dev, self.meant, want_var=False)
+        return mean, eng.predict_cov_device(xs_dev)
+
+    def estimate_cross_cov(self, x_a, x_b):
+        """Predictive covariance (ma, mb) between the rows of x_a and those of x_b, with the noise term of
+        cov_matrix_ij(x_a, x_b) of the covariance class."""
+        self._no_sparse("estimate_cross_cov")
+        xa = self._queries(x_a) if np.size(x_a) else np.zeros((0, self.d))
+        xb = self._queries(x_b) if np.size(x_b) else np.zeros((0, self.d))
+        if not xa.shape[0] or not xb.shape[0]:
+            return np.zeros((xa.shape[0], xb.shape[0]))
+        eng = self._engine()
+        if getattr(self.cov, "_KIND", None) is None:
+            ka = eng.to_device(np.asarray(self.cov.cov_matrix_ij(xa, self.x, self.theta_min), dtype=np.float64))
+            kb = eng.to_device(np.asarray(self.cov.cov_matrix_ij(xb, self.x, self.theta_min), dtype=np.float64))
+            prior = eng.to_device(np.asarray(self.cov.cov_matrix_ij(xa, xb, self.theta_min), dtype=np.float64))
+            cov = eng.predict_cov_cross_device(ka, kb, prior)
+        else:
+            cov = eng.predict_cov_device(eng.to_device(xa), eng.to_device(xb))
+        return cov.cpu().numpy()
+
     def estimate(self, x_star):
         """Mean and variance at one point (reference GaussianProcess.py:94-111)."""
         m, v = self.estimate_many(self._queries(np.atleast_2d(np.asarray(x_star, dtype=np.float64))))

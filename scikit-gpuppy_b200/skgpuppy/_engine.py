@@ -241,22 +241,67 @@ class Engine(object):
                                                int(want_var)), "gpk_predict")
         return mean, var
 
-    def predict_cross_device(self, Ks_dev, prior_dev, meant):
-        """Prediction from a caller-built m x n cross covariance and the m prior variances (gpk_predict_cross)."""
+    def predict_cross_device(self, Ks_dev, prior_dev, meant, want_var=True):
+        """Prediction from a caller-built m x n cross covariance and the m prior variances (gpk_predict_cross).
+        want_var False: means only (prior_dev may be None, the variance GEMM is skipped) and None for the variances."""
         torch = self.torch
         if Ks_dev.dim() != 2:
             raise ValueError("the cross covariance must be a (m, %d) tensor" % self.n)
         m = int(Ks_dev.shape[0])
         Ks_dev = self._dev_arg(Ks_dev, (m, self.n), "cross covariance")
-        prior_dev = self._dev_arg(prior_dev, (m,), "prior variances")
         mean = torch.empty((m,), dtype=torch.float64, device=self.device)
-        var = torch.empty((m,), dtype=torch.float64, device=self.device)
+        var = None
+        if want_var:
+            prior_dev = self._dev_arg(prior_dev, (m,), "prior variances")
+            var = torch.empty((m,), dtype=torch.float64, device=self.device)
         if m:
             with torch.cuda.device(self.device):
                 self._bind_stream()
-                nat.check(self.lib.gpk_predict_cross(self.h, nat.ptr(Ks_dev), self.n, m, nat.ptr(prior_dev), float(meant),
+                nat.check(self.lib.gpk_predict_cross(self.h, nat.ptr(Ks_dev), self.n, m,
+                                                     nat.ptr(prior_dev) if want_var else None, float(meant),
                                                      nat.ptr(mean), nat.ptr(var)), "gpk_predict_cross")
         return mean, var
+
+    def _rows_arg(self, t, ncols, what):
+        """A caller-supplied (m, ncols) device tensor and its m."""
+        if not isinstance(t, self.torch.Tensor) or t.dim() != 2:
+            raise ValueError("%s must be a 2-d (m, %d) tensor" % (what, ncols))
+        m = int(t.shape[0])
+        return self._dev_arg(t, (m, ncols), what), m
+
+    def predict_cov_device(self, xa_dev, xb_dev=None):
+        """Joint predictive covariance k(A, B) + noise - k(A, x) K^-1 k(x, B) as an (ma, mb) CUDA tensor
+        (gpk_predict_cov). xb_dev None: B = A, exactly symmetric, with the noise of cov_matrix(A)."""
+        torch = self.torch
+        xa_dev, ma = self._rows_arg(xa_dev, self.d, "queries A")
+        mb = ma
+        if xb_dev is not None:
+            xb_dev, mb = self._rows_arg(xb_dev, self.d, "queries B")
+        out = torch.empty((ma, mb), dtype=torch.float64, device=self.device)
+        if ma and mb:
+            with torch.cuda.device(self.device):
+                self._bind_stream()
+                nat.check(self.lib.gpk_predict_cov(self.h, nat.ptr(xa_dev), ma, nat.ptr(xb_dev), mb, nat.ptr(out), mb),
+                          "gpk_predict_cov")
+        return out
+
+    def predict_cov_cross_device(self, Ka_dev, Kb_dev, prior_dev):
+        """Joint predictive covariance from caller-built cross covariances Ka (ma, n), Kb (mb, n) or None for B = A,
+        and the prior block k(A, B) with its noise (ma, mb) (gpk_predict_cov_cross); an (ma, mb) CUDA tensor."""
+        torch = self.torch
+        Ka_dev, ma = self._rows_arg(Ka_dev, self.n, "cross covariance A")
+        mb = ma
+        if Kb_dev is not None:
+            Kb_dev, mb = self._rows_arg(Kb_dev, self.n, "cross covariance B")
+        prior_dev = self._dev_arg(prior_dev, (ma, mb), "prior covariance")
+        out = torch.empty((ma, mb), dtype=torch.float64, device=self.device)
+        if ma and mb:
+            with torch.cuda.device(self.device):
+                self._bind_stream()
+                nat.check(self.lib.gpk_predict_cov_cross(self.h, nat.ptr(Ka_dev), self.n, ma, nat.ptr(Kb_dev), self.n, mb,
+                                                         nat.ptr(prior_dev), mb, nat.ptr(out), mb),
+                          "gpk_predict_cov_cross")
+        return out
 
     def _ga_args(self, U_dev, S_dev, sigma_full):
         if U_dev.dim() != 2:
