@@ -164,6 +164,22 @@ int gpk_predict_cov_cross(gpk_handle h, const double* Ka_dev, int64_t lda, int64
                           const double* prior_dev, int64_t ldp, double* cov_dev, int64_t ldc);
 
 /*
+ * Gradients of the predictive mean and variance with respect to the query point (both device families):
+ *   mean[q] and var[q] as gpk_predict (noise included), dmean[q*d + k] = d mean[q] / d x*_qk = D_k . alpha,
+ *   dvar[q*d + k] = d var[q] / d x*_qk = -2 (X k*_q) . (X D_k),   D_k,i = d k(x*_q, x_i) / d x*_qk,
+ * with k*_q the row gpk_predict builds (prior k(x*, x*) is constant for both families).
+ * D is the true derivative: the reference's get_Jacobian (Covariance.py:676-689) has the opposite sign. Noise is a jump,
+ * not a slope: the vt added where a query coincides with a training point (periodic family, and the scalar rule of the
+ * Gaussian covariance) is left out of D. var_dev and dvar_dev: both NULL skips the O(n^2)
+ * product (rows and dots with alpha only); one of them NULL returns -2. Needs gpk_factorize (theta state), like
+ * gpk_predict. m == 0 does nothing.
+ * Workspace: one batch of d + 1 rows per query and, with the variances, its V^T (plus its residues on the INT8 route);
+ * if that does not fit the call returns -4 before any work is queued (byte counts in gpk_last_error()).
+ */
+int gpk_predict_grad(gpk_handle h, const double* xs_dev, int64_t m, double meant, double* mean_dev, double* var_dev,
+                     double* dmean_dev, double* dvar_dev);
+
+/*
  * Girard Gaussian approximation, batched over Q queries (UncertaintyPropagationApprox.propagate_GA,
  * UncertaintyPropagation2.pyx:266-299 with :208-257). U: Q x d means. S: Q x d (diagonal of Sigma_x) or,
  * with sigma_full, Q x d x d. Includes the equality-noise quirk of the scalar covariance (Covariance.py:451).

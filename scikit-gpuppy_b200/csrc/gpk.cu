@@ -35,7 +35,8 @@ struct Handle {
   double* colsq = nullptr; size_t colsq_elems = 0;    // [nbi][rows]
   double* pairdot = nullptr;                          // [nbi][rows/2]
   double* dots = nullptr; size_t dots_elems = 0;      // [rows]
-  double* V = nullptr; size_t V_elems = 0;            // gpk_predict_cov: rows of V^T = G X^T of both query sets
+  double* V = nullptr; size_t V_elems = 0;            // gpk_predict_cov: rows of V^T = G X^T of both query sets;
+                                                      // gpk_predict_grad: V^T of one batch
   double* C = nullptr; size_t C_elems = 0;            // gpk_predict_cov: padded output block
   long batch_rows = 0;                                // user cap on rows per batch (0 = default)
   SEHyper hyp;
@@ -1102,6 +1103,69 @@ int gpk_predict_cov_cross(gpk_handle h, const double* Ka, int64_t lda, int64_t m
     return -2;
   }
   return predict_cov_impl(hh, nullptr, Ka, lda, ma, nullptr, Kb, ldb, mb, prior, ldp, cov, ldc);
+}
+
+// Gradients of the predictive mean and variance at the query points xq (gpk_predict_grad). Each query owns P = d + 1
+// rows of G: k* from the family's tile kernel (leading dimension P npad, so the means are those of gpk_predict), then
+// D_1 .. D_d from grad_build_kernel; a batch holds whole queries. One rows_dot_kernel gives the means and their
+// gradients. With var: V^T = G X^T through the store product, group_dots_kernel forms V_0 . V_r per query, and
+// grad_finalize_kernel writes var = v + vt - |V_0|^2, dvar_k = -2 V_0 . V_k. Every allocation precedes the work.
+static int predict_grad_impl(Handle* h, const double* xq, long m, double meant, double* mean, double* var,
+                             double* dmean, double* dvar) {
+  const int npad = h->npad, n = h->n, d = h->d, P = d + 1, nbi = npad / TILE;
+  long qb_max = batch_rows_for(h, m * (long)P) / P;
+  if (qb_max < 1) qb_max = 1;
+  const long rows_max = round_up_l(qb_max * P, TILE);
+  if (var) GPK_TRY(ensure_route(h));
+  const size_t res_bytes = var && h->oz_on ? (size_t)h->oz.S * rows_max * npad : 0;
+  if (ensure_query_ws(h, rows_max) != 0 ||
+      (var && (ensure(&h->V, &h->V_elems, (size_t)rows_max * npad) != 0 ||
+               (h->oz_on && (h->ozq.ensure(res_bytes, (size_t)rows_max, (size_t)rows_max) != 0 ||
+                             ensure_query_planes(h, rows_max, npad) != 0))))) {
+    cudaGetLastError();   // the failed allocation is reported here, not by the next call
+    snprintf(g_err, sizeof(g_err),
+             "predictive gradient at n=%d, d=%d: %.2f GB of query batch + %.2f GB of V^T batch + %.2f GB of its residues "
+             "do not fit on the device",
+             n, d, 8.0 * rows_max * npad / 1e9, var ? 8.0 * rows_max * npad / 1e9 : 0.0, (double)res_bytes / 1e9);
+    return -4;
+  }
+  for (long q0 = 0; q0 < m; q0 += qb_max) {
+    const long qb = (m - q0) < qb_max ? m - q0 : qb_max;
+    const long rows = round_up_l(qb * P, TILE);
+    GPK_TRY(launch_se_tiles(xq + q0 * d, (int)qb, h->x, n, d, h->hyp, h->G, (long)P * npad, (int)qb, npad,
+                            noise_mode(h->kind, false), 0, 0, h->st));
+    GradArgs a;
+    a.xT = h->xT; a.ldxt = npad; a.xq = xq + q0 * d;
+    a.n = n; a.npad = npad; a.d = d; a.P = P; a.Q = (int)qb;
+    a.G = h->G; a.ldg = npad; a.rows_pad = (int)rows;
+    grad_build_kernel<<<dim3((npad + 255) / 256, (unsigned)(qb + (rows - qb * P))), 256, 0, h->st>>>(a, h->hyp);
+    GPK_LAUNCH_OK();
+    rows_dot_kernel<<<(unsigned)((qb * P + 7) / 8), 256, 0, h->st>>>(h->G, npad, (int)(qb * P), npad, h->alpha, h->dots);
+    GPK_LAUNCH_OK();
+    if (var) {
+      GPK_TRY(quad_forms(h, rows, h->V));
+      group_dots_kernel<<<dim3((unsigned)nbi, (unsigned)qb), 256, 0, h->st>>>(h->V, npad, P, h->colsq, rows);
+      GPK_LAUNCH_OK();
+    }
+    grad_finalize_kernel<<<(unsigned)((qb * P + 255) / 256), 256, 0, h->st>>>(
+        h->dots, var ? h->colsq : nullptr, rows, nbi, (int)qb, d, meant, h->hyp.v + h->hyp.vt, mean + q0, dmean + q0 * d,
+        var ? var + q0 : nullptr, dvar ? dvar + q0 * d : nullptr);
+    GPK_LAUNCH_OK();
+  }
+  return 0;
+}
+
+int gpk_predict_grad(gpk_handle h, const double* xs, int64_t m, double meant, double* mean, double* var, double* dmean,
+                     double* dvar) {
+  H_OR_FAIL(h);
+  if (!hh->factored || hh->matrix_state) { snprintf(g_err, sizeof(g_err), "not factored from theta"); return -2; }
+  if (m < 0) { snprintf(g_err, sizeof(g_err), "gpk_predict_grad: negative query count"); return -2; }
+  if (m == 0) return 0;
+  if (!xs || !mean || !dmean || (var == nullptr) != (dvar == nullptr)) {
+    snprintf(g_err, sizeof(g_err), "gpk_predict_grad: bad query or output argument (var and dvar go together)");
+    return -2;
+  }
+  return predict_grad_impl(hh, xs, m, meant, mean, var, dmean, dvar);
 }
 
 static int propagate_impl(gpk_handle h, const double* U, const double* S, int64_t Q, int sigma_full, double meant,

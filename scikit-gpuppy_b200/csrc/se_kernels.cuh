@@ -412,6 +412,102 @@ __global__ void __launch_bounds__(256) predict_var_kernel(const double* __restri
   var[q] = (prior ? prior[q] : vpvt) - s;
 }
 
+// ---------------------------------------------------------------------------------------------
+// Gradients of the predictive mean and variance (gpk_predict_grad). Query q of a batch owns the P = d + 1 rows
+// q*P .. q*P + d of G: row q*P is k*_q (the family's tile kernel, as in gpk_predict), row q*P + 1 + k is
+//   D_k,i = d k(x*_q, x_i) / d x*_qk,   delta = x*_qk - x_ik,
+//   Gaussian  -w_k delta E_i
+//   periodic  -E_i (w_k delta + w2_k (pi/p_k) sin(pi delta/p_k) cos(pi delta/p_k))
+// the true derivative (the reference's get_Jacobian, Covariance.py:676-689, has the opposite sign). E_i is the
+// covariance without noise: the vt added where two points coincide is a jump, not a slope.
+struct GradArgs {
+  const double* xT; long ldxt;  // x transposed: xT[k*ldxt + i]
+  const double* xq;             // [Q][d] query points of the batch
+  int n, npad, d, P, Q;
+  double* G; long ldg;
+  int rows_pad;                 // rows of G to clear beyond Q*P
+};
+
+__global__ void __launch_bounds__(256) grad_build_kernel(GradArgs p, SEHyper h) {
+  const int q = blockIdx.y;
+  const int i = blockIdx.x * 256 + threadIdx.x;
+  if (i >= p.npad) return;
+  if (q >= p.Q) {
+    // padding rows (beyond Q*P): zero
+    const long row = (long)p.Q * p.P + (q - p.Q);
+    if (row < p.rows_pad) p.G[row * p.ldg + i] = 0.0;
+    return;
+  }
+  double* g = p.G + ((long)q * p.P + 1) * p.ldg + i;
+  if (i >= p.n) {
+    for (int k = 0; k < p.d; ++k) g[(long)k * p.ldg] = 0.0;
+    return;
+  }
+  const double* u = p.xq + (long)q * p.d;
+  const bool per = h.kind == KIND_PERIODIC;
+  double dist = 0.0;
+  for (int k = 0; k < p.d; ++k) {
+    const double df = u[k] - p.xT[(long)k * p.ldxt + i];
+    dist = fma(h.w[k] * df, df, dist);
+    if (per) {
+      const double s = sin(h.pf[k] * df);
+      dist = fma(h.w2[k] * s, s, dist);
+    }
+  }
+  const double E = h.v * exp(-0.5 * dist);
+  for (int k = 0; k < p.d; ++k) {
+    const double df = u[k] - p.xT[(long)k * p.ldxt + i];
+    double s = h.w[k] * df;
+    if (per) {
+      double sn, cs;
+      sincos(h.pf[k] * df, &sn, &cs);
+      s = fma(h.w2[k] * h.pf[k] * sn, cs, s);
+    }
+    g[(long)k * p.ldg] = -s * E;
+  }
+}
+
+// part[b][q*P + r] = sum over columns 128b .. 128b+127 of V_0 V_r, V_r = row q*P + r of V^T (ld ldv): one CTA per
+// (column tile, query) reads the query's P rows once; warp w takes rows w, w + 8, ...
+__global__ void __launch_bounds__(256) group_dots_kernel(const double* __restrict__ Vt, long ldv, int P,
+                                                         double* __restrict__ part, long ldo) {
+  __shared__ double v0[TILE];
+  const int b = blockIdx.x, q = blockIdx.y;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const double* V = Vt + (long)q * P * ldv + (long)b * TILE;
+  if (threadIdx.x < TILE) v0[threadIdx.x] = V[threadIdx.x];
+  __syncthreads();
+  for (int r = warp; r < P; r += 8) {
+    const double* Vr = V + (long)r * ldv;
+    double s = 0.0;
+#pragma unroll
+    for (int c = lane; c < TILE; c += 32) s = fma(v0[c], Vr[c], s);
+    s = warp_sum(s);
+    if (lane == 0) part[(long)b * ldo + (long)q * P + r] = s;
+  }
+}
+
+// mean[q] = dots[q*P] (+ meant), dmean[q][k] = dots[q*P + 1 + k]; with part (column-tile partials of group_dots_kernel):
+// var[q] = v + vt - |V_0|^2, dvar[q][k] = -2 V_0 . V_{1+k}
+__global__ void __launch_bounds__(256) grad_finalize_kernel(const double* __restrict__ dots,
+                                                            const double* __restrict__ part, long ldo, int nbi, int Q,
+                                                            int d, double meant, double vpvt, double* __restrict__ mean,
+                                                            double* __restrict__ dmean, double* __restrict__ var,
+                                                            double* __restrict__ dvar) {
+  const int idx = blockIdx.x * 256 + threadIdx.x;
+  const int P = d + 1;
+  if (idx >= Q * P) return;
+  const int q = idx / P, r = idx % P;
+  const double a = dots[idx];
+  if (r == 0) mean[q] = meant != 0.0 ? a + meant : a;
+  else dmean[(long)q * d + r - 1] = a;
+  if (!part) return;
+  double s = 0.0;
+  for (int b = 0; b < nbi; ++b) s += part[(long)b * ldo + idx];
+  if (r == 0) var[q] = vpvt - s;
+  else dvar[(long)q * d + r - 1] = -2.0 * s;
+}
+
 __global__ void __launch_bounds__(256) add_scalar_kernel(double* __restrict__ y, int len, double a) {
   const int i = blockIdx.x * 256 + threadIdx.x;
   if (i < len) y[i] += a;

@@ -212,6 +212,31 @@ class GaussianProcess(object):
             cov = eng.predict_cov_device(eng.to_device(xa), eng.to_device(xb))
         return cov.cpu().numpy()
 
+    # -- gradients with respect to the query points (an addition: the reference differentiates its mean numerically) ---
+    def _grad_kind(self, what):
+        self._no_sparse(what)
+        if getattr(self.cov, "_KIND", None) is None:
+            raise NotImplementedError("%s: %s is built on the host and has no derivative in x on the device"
+                                      % (what, type(self.cov).__name__))
+
+    def estimate_many_grad(self, x_stars, want_var=True):
+        """Means (m,), variances (m,) and their gradients with respect to the query points, dmean (m, d) and dvar (m, d),
+        at the rows of x_stars. Means and variances are those of estimate_many (noise included); the gradients are the
+        true derivatives of the smooth part (the noise added where a query equals a training point is a jump). want_var
+        False: the variances and their gradients are None and the variance product is skipped."""
+        self._grad_kind("estimate_many_grad")
+        if np.size(x_stars) == 0:
+            dz = np.zeros((0, self.d))
+            return np.zeros(0), (np.zeros(0) if want_var else None), dz, (dz.copy() if want_var else None)
+        xs = self._queries(x_stars)
+        out = self.estimate_many_grad_device(self._engine().to_device(xs), want_var=want_var)
+        return tuple(None if o is None else o.cpu().numpy() for o in out)
+
+    def estimate_many_grad_device(self, xs_dev, want_var=True):
+        """Same on device-resident queries; returns CUDA tensors (mean, var, dmean, dvar)."""
+        self._grad_kind("estimate_many_grad_device")
+        return self._engine().predict_grad_device(xs_dev, self.meant, want_var=want_var)
+
     def estimate(self, x_star):
         """Mean and variance at one point (reference GaussianProcess.py:94-111)."""
         m, v = self.estimate_many(self._queries(np.atleast_2d(np.asarray(x_star, dtype=np.float64))))

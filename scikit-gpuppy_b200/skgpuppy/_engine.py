@@ -303,6 +303,25 @@ class Engine(object):
                           "gpk_predict_cov_cross")
         return out
 
+    def predict_grad_device(self, xs_dev, meant, want_var=True):
+        """(mean (m,), var (m,), dmean (m, d), dvar (m, d)) as CUDA tensors (gpk_predict_grad): the predictive moments
+        and their derivatives with respect to the query points. want_var False: var and dvar are None and the variance
+        product is skipped."""
+        torch = self.torch
+        xs_dev, m = self._rows_arg(xs_dev, self.d, "queries")
+        mean = torch.empty((m,), dtype=torch.float64, device=self.device)
+        dmean = torch.empty((m, self.d), dtype=torch.float64, device=self.device)
+        var = dvar = None
+        if want_var:
+            var = torch.empty((m,), dtype=torch.float64, device=self.device)
+            dvar = torch.empty((m, self.d), dtype=torch.float64, device=self.device)
+        if m:
+            with torch.cuda.device(self.device):
+                self._bind_stream()
+                nat.check(self.lib.gpk_predict_grad(self.h, nat.ptr(xs_dev), m, float(meant), nat.ptr(mean), nat.ptr(var),
+                                                    nat.ptr(dmean), nat.ptr(dvar)), "gpk_predict_grad")
+        return mean, var, dmean, dvar
+
     def _ga_args(self, U_dev, S_dev, sigma_full):
         if U_dev.dim() != 2:
             raise ValueError("U must be a (Q, %d) tensor" % self.d)

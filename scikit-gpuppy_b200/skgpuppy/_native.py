@@ -42,6 +42,7 @@ SIGNATURES = {
     "gpk_predict_cross": (ctypes.c_int, [vp, vp, i64, i64, vp, ctypes.c_double, vp, vp]),
     "gpk_predict_cov": (ctypes.c_int, [vp, vp, i64, vp, i64, vp, i64]),
     "gpk_predict_cov_cross": (ctypes.c_int, [vp, vp, i64, i64, vp, i64, i64, vp, i64, vp, i64]),
+    "gpk_predict_grad": (ctypes.c_int, [vp, vp, i64, ctypes.c_double, vp, vp, vp, vp]),
     "gpk_propagate_ga": (ctypes.c_int, [vp, vp, vp, i64, ctypes.c_int, ctypes.c_double, vp, vp]),
     "gpk_propagate_ga_parts": (ctypes.c_int, [vp, vp, vp, i64, ctypes.c_int, vp, vp]),
     "gpk_propagate_exact": (ctypes.c_int, [vp, vp, vp, vp, vp, i64, ctypes.c_double, vp, vp]),
