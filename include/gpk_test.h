@@ -38,6 +38,13 @@ int gpk_test_oz_gemm(const double* A_dev, int64_t lda, int transA, int lowerA, c
  * (exact integer sums). Other values leave the setting unchanged. Returns the setting. */
 int gpk_test_position_lock(int on);
 
+/* Unwritten-memory check (calling thread only): while byte != 0, every device buffer the library allocates (handle
+ * buffers, query and gradient scratch, INT8 residue workspaces) is filled with `byte` right after allocation; switching
+ * it on also refills the device's position-lock scratch. 0xFF makes every double a NaN, 0x7F every double 1.4e306.
+ * Outputs must not depend on it. Returns the KiB of allocations filled since the previous call (so that a test can
+ * check the fill took place; the refill of the position-lock scratch is not counted), or -1 on a CUDA error. */
+int gpk_test_poison(int byte);
+
 /* INT8 route (calling thread only): 1 = T = L21 X11 of each node overlaps the right sub-tree on its own stream when
  * the handle has the memory (default), 0 = every product on one stream; any other value leaves it unchanged. Takes
  * effect at the next factorisation (the workspaces follow at the next gpk_set_route). Returns the setting. */

@@ -167,6 +167,7 @@ static int ensure(double** p, size_t* have, size_t need) {
   *have = 0;
   GPK_CUDA_OK(cudaMalloc((void**)p, need * sizeof(double)));
   *have = need;
+  GPK_CUDA_OK(poison_fill(*p, need * sizeof(double)));
   return 0;
 }
 
@@ -538,6 +539,14 @@ static int create_fill(Handle* h, int64_t n, int64_t d, double* Xbuf, double* Wb
   GPK_CUDA_OK(cudaMalloc((void**)&h->dL, np * sizeof(double)));
   GPK_CUDA_OK(cudaMalloc((void**)&h->scal, 3 * sizeof(double)));
   GPK_CUDA_OK(cudaMalloc((void**)&h->info, sizeof(int)));
+  if (h->own_X) GPK_CUDA_OK(poison_fill(h->X, np * np * sizeof(double)));
+  if (h->own_W) GPK_CUDA_OK(poison_fill(h->W, np * np * sizeof(double)));
+  GPK_CUDA_OK(poison_fill(h->x, (size_t)n * d * sizeof(double)));
+  GPK_CUDA_OK(poison_fill(h->xT, (size_t)d * np * sizeof(double)));
+  GPK_CUDA_OK(poison_fill(h->y, np * sizeof(double)));
+  GPK_CUDA_OK(poison_fill(h->dL, np * sizeof(double)));
+  GPK_CUDA_OK(poison_fill(h->scal, 3 * sizeof(double)));
+  GPK_CUDA_OK(poison_fill(h->info, sizeof(int)));
   GPK_CUDA_OK(cudaMemset(h->t, 0, np * sizeof(double)));
   GPK_CUDA_OK(cudaMemset(h->alpha, 0, np * sizeof(double)));
   {
@@ -1353,6 +1362,16 @@ int gpk_test_oz_gemm(const double* A, int64_t lda, int transA, int lowerA, const
 int gpk_test_position_lock(int on) {
   if (on >= 0 && on <= 2) oz::g_position_lock = on;
   return oz::g_position_lock;
+}
+
+int gpk_test_poison(int byte) {
+  const size_t kib = g_poison_bytes >> 10;
+  g_poison_bytes = 0;
+  g_poison = byte & 0xff;
+  int*& spill = oz::g_spill_dev[current_device_slot()];
+  if (spill) GPK_CUDA_OK(poison_fill(spill, oz::SPILL_BYTES));
+  g_poison_bytes = 0;   // the count covers allocations only
+  return kib > INT_MAX ? INT_MAX : (int)kib;
 }
 
 int gpk_test_overlap(int on) {

@@ -33,6 +33,17 @@ extern thread_local long g_launch_count;
 extern thread_local bool g_prof_on;
 void prof_push(cudaEvent_t a, cudaEvent_t b);
 
+// gpk_test_poison: while nonzero, every device buffer the library allocates is filled with this byte (test hook: a
+// read of memory the library never wrote then shows in the results)
+inline thread_local int g_poison = 0;
+inline thread_local size_t g_poison_bytes = 0;   // bytes filled since the last gpk_test_poison call
+inline cudaError_t poison_fill(void* p, size_t bytes) {
+  if (!g_poison || !p || !bytes) return cudaSuccess;
+  g_poison_bytes += bytes;
+  const cudaError_t e = cudaMemset(p, g_poison, bytes);
+  return e == cudaSuccess ? cudaDeviceSynchronize() : e;
+}
+
 #define GPK_CUDA_OK(expr)                                                         \
   do {                                                                            \
     cudaError_t _e = (expr);                                                      \

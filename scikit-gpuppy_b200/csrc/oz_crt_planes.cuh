@@ -382,7 +382,13 @@ __global__ void __launch_bounds__(256, 4) oz_crt_reconstruct_kernel(const __grid
     const unsigned long long t2 = ((unsigned long long)acc[x][5] << 16) + acc[x][4] + (t1 >> 32);
     const long long hi = (long long)((t2 << 32) | (t1 & 0xffffffffull));
     const double frac = fma((double)hi, 4294967296.0, (double)(uint32_t)t0);   // signed 96-bit integer, 53 leading bits
-    v[x] = col_ok ? sa * p.scB[gcol + x] * frac : 0.0;
+    // (sa scB) frac rounds once. When sa scB underflows (eA + eB - 2 bits + log2 p_scaled < -1022: subnormal, or 0 below
+    // about -1074) it has lost bits while the value itself may be normal: (sa frac) scB rounds once too there (sa frac is
+    // normal, scB a power of two), and gives the same bits wherever both orders are exact. sa and scB are never 0 for a
+    // valid row and column, so the test is on the range, not on sab itself.
+    const double sab = col_ok ? sa * p.scB[gcol + x] : 0.0;
+    v[x] = col_ok ? sab * frac : 0.0;
+    if (row_ok && col_ok && fabs(sab) < 2.2250738585072014e-308) v[x] = sa * frac * p.scB[gcol + x];
   }
   if (EPI == OZ_EPI_STORE) {
     if (row_ok && col_ok) {

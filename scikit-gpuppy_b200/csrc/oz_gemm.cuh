@@ -202,49 +202,55 @@ __device__ __forceinline__ size_t slice_offset(int rows, int K, int p, int r, in
          ((size_t)(r & 127) << 7) + (size_t)(k & 127);
 }
 
-// mx[r] = bits of max_k |operand(r,k)|  (non-negative doubles order like their bit patterns)
+// mx[r] = bits of max_k |operand(r,k)| over the valid tiles, or of +Inf if one of them is not finite. The maximum is
+// taken on the bit patterns: non-negative doubles order like them, and |NaN| orders above +Inf (fmax would drop it).
+constexpr unsigned long long OZ_INF_BITS = 0x7ff0000000000000ull;
+__device__ __forceinline__ unsigned long long oz_abs_bits(double x) {
+  return (unsigned long long)__double_as_longlong(x) & 0x7fffffffffffffffull;
+}
 __global__ void __launch_bounds__(256) oz_absmax_rows_kernel(const double* __restrict__ src, long ld, int K, int lower,
                                                              unsigned long long* __restrict__ mx) {
-  __shared__ double red[8];
+  __shared__ unsigned long long red[8];
   const int r = blockIdx.x;
   const int kend = lower ? min(K, ((r >> 7) + 1) << 7) : K;
   const double* row = src + (long)r * ld;
-  double m = 0.0;
-  for (int k = threadIdx.x; k < kend; k += 256) m = fmax(m, fabs(row[k]));
+  unsigned long long m = 0ull;
+  for (int k = threadIdx.x; k < kend; k += 256) m = max(m, oz_abs_bits(row[k]));
 #pragma unroll
-  for (int o = 16; o > 0; o >>= 1) m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
+  for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(0xffffffffu, m, o));
   if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = m;
   __syncthreads();
   if (threadIdx.x == 0) {
 #pragma unroll
-    for (int i = 0; i < 8; ++i) m = fmax(m, red[i]);
-    mx[r] = (unsigned long long)__double_as_longlong(m);
+    for (int i = 0; i < 8; ++i) m = max(m, red[i]);
+    mx[r] = min(m, OZ_INF_BITS);
   }
 }
 // transposed operand: rows of the operand are columns of the source. grid (rows/32, ceil(K/1024)), 256 threads.
 __global__ void __launch_bounds__(256) oz_absmax_cols_kernel(const double* __restrict__ src, long ld, int K, int lower,
                                                              unsigned long long* __restrict__ mx) {
-  __shared__ double red[8][32];
+  __shared__ unsigned long long red[8][32];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int r = blockIdx.x * 32 + lane;
   const int k0 = blockIdx.y * 1024, k1 = min(K, k0 + 1024);
   const int kfirst = lower ? ((r >> 7) << 7) : 0;
-  double m = 0.0;
+  unsigned long long m = 0ull;
   for (int k = k0 + w; k < k1; k += 8)
-    if (k >= kfirst) m = fmax(m, fabs(src[(long)k * ld + r]));
+    if (k >= kfirst) m = max(m, oz_abs_bits(src[(long)k * ld + r]));
   red[w][lane] = m;
   __syncthreads();
   if (w == 0) {
 #pragma unroll
-    for (int i = 1; i < 8; ++i) m = fmax(m, red[i][lane]);
-    atomicMax(mx + r, (unsigned long long)__double_as_longlong(m));
+    for (int i = 1; i < 8; ++i) m = max(m, red[i][lane]);
+    atomicMax(mx + r, min(m, OZ_INF_BITS));
   }
 }
 
-// exponent e with |x| < 2^e for every element of the row; rows that are zero (or not finite) get e = 0
+// exponent e with |x| < 2^e for every element of the row; rows that are zero (or not finite) get e = 0.
+// Rows whose maximum is below 2^-900 are flushed to zero: their elements scale below 2^(bits - 900 - 1) and round to 0.
 __device__ __forceinline__ int oz_row_exponent(unsigned long long bits) {
   const double m = __longlong_as_double((long long)bits);
-  if (!(m > 0.0) || !isfinite(m)) return 0;
+  if (!(m > 0.0) || bits >= OZ_INF_BITS) return 0;
   int e = ilogb(m) + 1;
   if (e < -900) e = -900;
   return e;
@@ -323,13 +329,15 @@ __global__ void __launch_bounds__(256) oz_residue_rows_kernel(const double* __re
   const int cpr = K >> 4;
   if (idx >= (long)rows * cpr) return;
   const int r = (int)(idx / cpr), ch = (int)(idx % cpr);
+  // a row with a non-finite element: scale NaN, residues zero, so the reconstruction makes the whole output row NaN
+  const bool finite = mx[r] < OZ_INF_BITS;
   const int e = oz_row_exponent(mx[r]);
-  if (ch == 0) sc[r] = ldexp(1.0, e - bits);
+  if (ch == 0) sc[r] = finite ? ldexp(1.0, e - bits) : __longlong_as_double(0x7ff8000000000000ll);
   const double scale = ldexp(1.0, bits - e);
   const int k0 = ch << 4;
   if (!oz_needed<0>(r, k0, lower, extra)) return;
   uint32_t lo[16], hi[16];
-  if (oz_valid<0>(r, k0, lower)) {
+  if (finite && oz_valid<0>(r, k0, lower)) {
     const double2* s2 = reinterpret_cast<const double2*>(src + (long)r * ld + k0);
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
@@ -354,12 +362,13 @@ __global__ void __launch_bounds__(256) oz_residue_cols_kernel(const double* __re
   const int r = blockIdx.x * 32 + lane;
   const int k0 = (blockIdx.y * 8 + w) * 16;
   if (k0 >= K) return;
+  const bool finite = mx[r] < OZ_INF_BITS;   // as in oz_residue_rows_kernel
   const int e = oz_row_exponent(mx[r]);
-  if (k0 == 0) sc[r] = ldexp(1.0, e - bits);
+  if (k0 == 0) sc[r] = finite ? ldexp(1.0, e - bits) : __longlong_as_double(0x7ff8000000000000ll);
   const double scale = ldexp(1.0, bits - e);
   if (!oz_needed<1>(r, k0, lower, extra)) return;
   uint32_t lo[16], hi[16];
-  const bool valid = oz_valid<1>(r, k0, lower);
+  const bool valid = finite && oz_valid<1>(r, k0, lower);
 #pragma unroll
   for (int i = 0; i < 16; ++i) oz_split(valid ? src[(long)(k0 + i) * ld + r] : 0.0, scale, lo[i], hi[i]);
   for (int p = 0; p < nmod; ++p)
@@ -447,6 +456,11 @@ inline int slice_operand(const double* src, long ld, int trans, int lower, Opera
   return 0;
 }
 
+// scratch of the position lock (oz_crt_planes_kernel): one slot per SM, shared by every launch on the device (a slot
+// belongs to the one CTA that is resident on that SM)
+inline int* g_spill_dev[GPK_MAX_DEVICES] = {};
+constexpr size_t SPILL_BYTES = (size_t)SPILL_SLOTS * BM * Q_BN * sizeof(int);
+
 thread_local int g_position_lock = 2;   // gpk_test_position_lock: 0 = lock on the modulus only, 1 = + split first modulus, 2 = + band-uniform k ranges
 
 // C = beta*C + alpha * A * B^T over the per-tile k range, from operands in residue form (A.K == B.K, A.S == B.S):
@@ -506,13 +520,16 @@ inline int gemm_sliced(const Operand& A, const Operand& B, double* C, long ldc, 
   // position counters (see oz_crt_planes_kernel): a fresh one per launch, launches on different streams may overlap
   static unsigned int* phase_dev_on[GPK_MAX_DEVICES] = {};
   unsigned int*& phase_dev = phase_dev_on[current_device_slot()];
-  if (!phase_dev) GPK_CUDA_OK(cudaMalloc((void**)&phase_dev, 64 * sizeof(unsigned int)));
+  if (!phase_dev) {
+    GPK_CUDA_OK(cudaMalloc((void**)&phase_dev, 64 * sizeof(unsigned int)));
+    GPK_CUDA_OK(poison_fill(phase_dev, 64 * sizeof(unsigned int)));
+  }
   static thread_local int phase_next = 0;
-  // scratch of the position lock (oz_crt_planes_kernel): one slot per SM, shared by every launch on the device (a slot
-  // belongs to the one CTA that is resident on that SM)
-  static int* spill_dev_on[GPK_MAX_DEVICES] = {};
-  int*& spill_dev = spill_dev_on[current_device_slot()];
-  if (!spill_dev) GPK_CUDA_OK(cudaMalloc((void**)&spill_dev, (size_t)SPILL_SLOTS * BM * Q_BN * sizeof(int)));
+  int*& spill_dev = g_spill_dev[current_device_slot()];
+  if (!spill_dev) {
+    GPK_CUDA_OK(cudaMalloc((void**)&spill_dev, SPILL_BYTES));
+    GPK_CUDA_OK(poison_fill(spill_dev, SPILL_BYTES));
+  }
   g.spill = g_position_lock ? spill_dev : nullptr;
   cudaEvent_t e0 = nullptr, e1 = nullptr;
   if (g_prof_on) {
@@ -591,6 +608,7 @@ struct Workspace {
     out = nullptr; out_cap = 0;
     if (cudaMalloc((void**)&out, bytes) != cudaSuccess) { cudaGetLastError(); out = nullptr; return -1; }
     out_cap = bytes;
+    if (poison_fill(out, bytes) != cudaSuccess) return -1;
     return 0;
   }
   int ensure(size_t bytes, size_t rows_total, size_t rows_max) {
@@ -599,18 +617,21 @@ struct Workspace {
       buf = nullptr; cap = 0;
       if (cudaMalloc((void**)&buf, bytes) != cudaSuccess) { cudaGetLastError(); buf = nullptr; return -1; }
       cap = bytes;
+      if (poison_fill(buf, bytes) != cudaSuccess) return -1;
     }
     if (rows_total > sc_cap) {
       if (sc) cudaFree(sc);
       sc = nullptr; sc_cap = 0;
       if (cudaMalloc((void**)&sc, rows_total * sizeof(double)) != cudaSuccess) { cudaGetLastError(); return -1; }
       sc_cap = rows_total;
+      if (poison_fill(sc, rows_total * sizeof(double)) != cudaSuccess) return -1;
     }
     if (rows_max > mx_cap) {
       if (mx) cudaFree(mx);
       mx = nullptr; mx_cap = 0;
       if (cudaMalloc((void**)&mx, rows_max * sizeof(unsigned long long)) != cudaSuccess) { cudaGetLastError(); return -1; }
       mx_cap = rows_max;
+      if (poison_fill(mx, rows_max * sizeof(unsigned long long)) != cudaSuccess) return -1;
     }
     return 0;
   }

@@ -61,6 +61,7 @@ TEST_SIGNATURES = {
                                         i64, i64, i64, ctypes.c_double, ctypes.c_double, ctypes.c_int, ctypes.c_int,
                                         ctypes.c_int, i64, ctypes.c_int, ctypes.POINTER(ctypes.c_float), vp]),
     "gpk_test_overlap": (ctypes.c_int, [ctypes.c_int]),
+    "gpk_test_poison": (ctypes.c_int, [ctypes.c_int]),
     "gpk_test_position_lock": (ctypes.c_int, [ctypes.c_int]),
     "gpk_profile": (ctypes.c_int, [ctypes.c_int]),
     "gpk_profile_read": (ctypes.c_int, [c_double_p, ctypes.POINTER(i64), ctypes.POINTER(i64), c_double_p]),
